@@ -10,9 +10,10 @@ flow past a cylinder, D2Q9 BGK, compressible equilibrium, immersed-boundary cyli
 anti-bounce-back inlet/outlet rows, specular side columns (test/cylinder_test.cpp of the reference), 8192 x 8192 nodes PER
 GPU (weak scaling: the global grid is (8192 N) x 8192, slab-decomposed along axis 0 like test/decompose_domain.cpp).
 
-The K-step block is timed with CUDA events on the domain's stream (max over ranks); a block shorter than 0.2 s is
-repeated (at least 5 blocks and a quarter of a second of device time, at most 50; longer blocks: 3) and the MEDIAN block is reported — every block is
-exactly K steps.  Rank 0 prints ONE JSON line.  Beside the headline the same line carries
+After W warm-up steps (at least 4 where the step pair replays as a CUDA graph: its capture takes 4), exactly K steps are
+timed as one block with CUDA events on the domain's stream (max over ranks).
+--dump-outputs DIR then writes what those steps left in the headline domain (see dump_outputs), so that two builds run
+with the same arguments can be compared output for output.  Rank 0 prints ONE JSON line.  Beside the headline the same line carries
   other_workloads  N = 1: every other BASELINE.json config at its named size (device-resident value + roofline of its
                    dominant kernel); every N: `mrtcg_rt_weak`, the MRT colour-gradient step at 8192 x 16384 nodes per GPU —
                    the model with two-row moment-plane halos — so that the 1 -> 8 GPU records hold a curve for it too
@@ -24,7 +25,6 @@ The CPU baseline (N = 1 only) runs after all GPU work, so no GPU idles in a coll
 import argparse
 import ctypes
 import json
-import math
 import os
 import subprocess
 import sys
@@ -37,7 +37,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "lattice-boltzmann-method_b200", "python"))
 
-FALLBACK_HBM_GBS = 6650.0        # /opt/skills/guides/B200_PROFILING.md
+FALLBACK_HBM_GBS = 6650.0        # B200 HBM3e bandwidth assumed where no MEASURED_PEAKS.json gives a measured one
 CSF_FUSED_DEFAULT = "1"          # the library's default for LBM_CSF_FUSED (csrc/lbm_two_phase.cu: the single pass, k_csf_staged)
 
 W9 = np.array([4 / 9] + [1 / 9] * 4 + [1 / 36] * 4)
@@ -129,7 +129,12 @@ def parse_args():
     ap.add_argument("--lib", default="", help="development: another build of the library (path) for an A/B run")
     ap.add_argument("--graph", default="auto", choices=["auto", "on", "off"],
                     help="replay the step pair as a CUDA graph (auto: grids up to 2^24 nodes on one GPU, where launches bound the step)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the headline's state after the timed steps to DIR/<name>.npy (float64, sampled nodes on large "
+                         "grids); the B200 arm only")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the state of the B200 arm's domain: it needs --impl b200")
     wl = WORKLOADS[args.workload]
     args.X = args.X or wl["X"]
     args.Y = args.Y or wl["Y"]
@@ -513,7 +518,7 @@ def measured_hbm_peak():
         with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as fh:
             return float(json.load(fh)["hbm_gbs"]), "measured (MEASURED_PEAKS.json)"
     except Exception:
-        return FALLBACK_HBM_GBS, "fallback (B200_PROFILING.md)"
+        return FALLBACK_HBM_GBS, "fallback (FALLBACK_HBM_GBS of bench.py)"
 
 
 def ncu_traffic_per_launch(workload, X, Y):
@@ -723,9 +728,33 @@ def want_graph(mode, X, Y, world):
     return mode == "on" or X * Y <= (1 << 24)
 
 
-def measure(ctx, workload, X, Y, steps, warmup, *, pin, with_e2e, graph_mode, sampler=None, cpu_sample=0):
-    """Device-resident MLUPS of one workload (median K-step block), the roofline of its dominant kernel and, for the
-    headline, the end-to-end figure through the C ABI with pinned host buffers."""
+DUMP_NODES = 1 << 17  # nodes written by --dump-outputs, over all ranks: at most 2 x 9 + 3 float64 values each, 22 MB
+
+
+def dump_outputs(ctx, case, out_dir):
+    """What a caller of lbm_step receives after the timed steps: the populations of every lattice (lbm_get_f, `f0`, `f1`)
+    and rho, u (lbm_get_moments of lattice 0), as float64 arrays of shape (nodes, components) over the slab's nodes in
+    row-major order.  A slab of more than DUMP_NODES / ranks nodes contributes a fixed, seeded, sorted sample of that many
+    nodes; rank 0 writes the ranks' rows one after the other."""
+    d, n = case.d, case.X * case.Y
+    k = DUMP_NODES // ctx.world
+    idx = np.arange(n) if n <= k else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    rho, u = d.get_moments(0)
+    out = {"rho": rho.reshape(n, 1)[idx], "u": u.reshape(n, 2)[idx]}
+    for lat in range(WORKLOADS[case.label]["nlat"]):
+        out[f"f{lat}"] = d.get_f(lat).reshape(n, 9)[idx]
+    if ctx.world > 1:
+        out = {name: ctx.gather_rows(a) for name, a in out.items()}
+    if ctx.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in out.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
+def measure(ctx, workload, X, Y, steps, warmup, *, pin, with_e2e, graph_mode, sampler=None, cpu_sample=0, dump_dir=""):
+    """Device-resident MLUPS of one workload (one block of exactly K steps), the roofline of its dominant kernel and, for
+    the headline, the end-to-end figure through the C ABI with pinned host buffers.  dump_dir: dump_outputs after the
+    timed block."""
     import types
 
     L, rank, world = ctx.L, ctx.rank, ctx.world
@@ -739,37 +768,33 @@ def measure(ctx, workload, X, Y, steps, warmup, *, pin, with_e2e, graph_mode, sa
     if world > 1:
         d.comm_check()  # every rank's setup agrees (grid, model, marker lists of bodies across cuts) or LBM_ERR_COMM — not a hang
     case.import_state()
-    d.step(warmup)
     graph = want_graph(graph_mode, X, Y, world)
+    # W warm-up steps in all; with the graph the last 4 of them reach the steady state and capture the pair (so at least 4)
+    d.step(max(warmup - 4, 0) if graph else warmup)
     if graph:
         d.use_graph(True)
-        d.step(4)  # reaches the steady state and captures the pair
+        d.step(4)
     ctx.barrier(d)
 
-    # ---- device-resident timed region: blocks of exactly K steps, CUDA events on the domain's stream
+    # ---- device-resident timed region: exactly K steps in one block, CUDA events on the domain's stream
     d.profile_enable(not graph)
     launches0 = d.kernel_launches()
-    block_ms, target = [], None
     if sampler is not None:
         sampler.mark_begin()
-    while target is None or len(block_ms) < target:
-        ctx.barrier(d)
-        d.step(steps)
-        d.synchronize()
-        block_ms.append(ctx.max_over_ranks(d.last_step_ms()))
-        if target is None:
-            # K steps shorter than 0.2 s: at least 5 blocks and about a quarter of a second of timed work; else 3 blocks
-            target = 3 if block_ms[0] >= 200.0 else int(min(50, max(5, math.ceil(250.0 / max(block_ms[0], 1e-3)))))
+    ctx.barrier(d)
+    d.step(steps)
+    d.synchronize()
+    ms = ctx.max_over_ranks(d.last_step_ms())
     ctx.barrier(d)
     if sampler is not None:
         sampler.mark_end()
-    nb = len(block_ms)
-    launches = (d.kernel_launches() - launches0) // nb
-    ms = float(np.median(block_ms))
-    prof_steps = steps * nb
+    launches = d.kernel_launches() - launches0
+    prof_steps = steps
+    if dump_dir:
+        dump_outputs(ctx, case, dump_dir)
     if graph:
         # the graph replays without per-kernel events: the dominant kernel's duration comes from one more K-step block of
-        # plain launches of the same kernel (same grid, same launch configuration), right after the timed blocks
+        # plain launches of the same kernel (same grid, same launch configuration), right after the timed block
         d.use_graph(False)
         d.profile_enable(True)
         d.step(steps)
@@ -845,12 +870,12 @@ def measure(ctx, workload, X, Y, steps, warmup, *, pin, with_e2e, graph_mode, sa
                 "share_of_step": (dom_ms / prof_steps) / (ms / steps),
                 "other_spans_ms_per_step": {k: v[0] / prof_steps for k, v in prof.items() if v[1] and k not in ("interior", "early_rows")},
                 "early_rows_ms_per_step": prof["early_rows"][0] / prof_steps,
-                "timed_in": ("one more K-step block of plain launches after the timed blocks (those replay a CUDA graph)" if graph
-                             else "the timed blocks themselves (CUDA events around every launch of the kernel, rank 0)"),
+                "timed_in": ("one more K-step block of plain launches after the timed block (that one replays a CUDA graph)" if graph
+                             else "the timed block itself (CUDA events around every launch of the kernel, rank 0)"),
                 "note": f"achieved = {B:.0f} B x nodes the dominant kernel owns per step / summed duration of its launches (single-phase "
                         "family: early rows then bulk rows, one after the other); listed nodes, stages, ghost rows and the IBM "
                         "pre-pass run on a side stream under the bulk launch"}
-    out = {"value": mlups, "ms_per_step": ms / steps, "steps": steps, "blocks": nb, "block_ms": [round(v, 4) for v in block_ms],
+    out = {"value": mlups, "ms_per_step": ms / steps, "steps": steps, "blocks": 1, "block_ms": [round(ms, 4)],
            "cuda_graph": graph, "grid_per_gpu": [X, Y], "global_grid": [case.Xg, Y], "gpu_launches": launches, "roofline": roofline,
            "e2e": e2e, "what": wl["what"], "reference_driver": wl["driver"]}
     d.close()
@@ -1060,7 +1085,7 @@ def run_b200_arm(args):
     if rank == 0:
         sampler.start()
     head = measure(ctx, args.workload, args.X, args.Y, args.steps, args.warmup, pin=True, with_e2e=not args.no_e2e,
-                   graph_mode=args.graph, sampler=sampler, cpu_sample=args.cpu_sample)
+                   graph_mode=args.graph, sampler=sampler, cpu_sample=args.cpu_sample, dump_dir=args.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
 
     # ---- the other configs (device-resident value + roofline), only beside the default headline
@@ -1099,7 +1124,7 @@ def run_b200_arm(args):
         "dtype": "f64", "data": "synthetic", "config": workload_config(args, world),
         "roofline": head["roofline"], "cpu_baseline": cpu_baseline, "e2e": head["e2e"], "gpu_launches": head["gpu_launches"],
         "clocks": clocks,
-        "timing": {"blocks": head["blocks"], "block_ms": head["block_ms"], "reported": "median block of exactly K steps",
+        "timing": {"blocks": head["blocks"], "block_ms": head["block_ms"], "reported": "one block of exactly K steps after W warm-up steps (at least 4 with the CUDA graph)",
                    "cuda_graph": head["cuda_graph"]},
         "other_workloads": others or None, "ring_parity": ring,
     }

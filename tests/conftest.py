@@ -11,7 +11,7 @@ sys.path.insert(0, os.path.join(ROOT, "lattice-boltzmann-method_b200", "python")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "ref: needs oracle/_ref (the compiled reference; built only where /root/reference exists)")
+    config.addinivalue_line("markers", "ref: needs oracle/_ref (the compiled reference; built only from a checkout of the original sources, see oracle/Makefile)")
 
 
 # TEST INFRASTRUCTURE: LBM_EMU=1 points the binding at tests/cpu_emu/_build/liblbm_b200_emu.so — the library's own CUDA

@@ -38,6 +38,31 @@ def test_reference_arm_line(workload):
     assert e["value"] == d["value"] and e["unit"] == d["unit"] and e["h2d_bytes_per_step"] == 0 and e["d2h_bytes_per_step"] == 0
 
 
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_state_after_exactly_warmup_plus_steps(tmp_path):
+    """--dump-outputs writes the headline's state after the timed block: two runs with the same number of warm-up + timed
+    steps write the same arrays, one more timed step changes them (warm-ups of at least 4: this grid replays a CUDA graph)"""
+    import numpy as np
+
+    if os.environ.get("LBM_EMU") == "1":
+        pytest.skip("bench.py's B200 arm needs a real device")
+    X, Y = 96, 64
+    dumps = []
+    for warmup, steps in ((6, 3), (5, 4), (5, 5)):
+        out = tmp_path / f"w{warmup}_k{steps}"
+        r = run(["--steps", str(steps), "--warmup", str(warmup), "--X", str(X), "--Y", str(Y), "--no-others", "--no-cpu-baseline",
+                 "--no-e2e", "--dump-outputs", str(out)])
+        assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-1500:]
+        d = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+        assert d["steps"] == steps and d["timing"]["blocks"] == 1
+        dumps.append({p.stem: np.load(p) for p in out.glob("*.npy")})
+    shapes = {"f0": (X * Y, 9), "rho": (X * Y, 1), "u": (X * Y, 2)}
+    assert {k: v.shape for k, v in dumps[0].items()} == shapes and all(v.dtype == np.float64 for v in dumps[0].values())
+    relerr = lambda a, b: float(np.abs(a - b).max() / np.abs(b).max())  # noqa: E731
+    assert all(relerr(dumps[1][k], dumps[0][k]) < 1e-12 for k in shapes)
+    assert relerr(dumps[2]["u"], dumps[0]["u"]) > 1e-9
+
+
 def test_b200_arm_needs_a_device():
     import torch
     if torch.cuda.is_available():

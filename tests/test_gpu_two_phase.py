@@ -153,10 +153,11 @@ def test_rk_droplet_vs_oracle_and_golden(orc):
             n += 1
         fr, fb = d.get_f(0), d.get_f(1)
         assert cases.relerr(fr, st["r_adv"]) < 1e-12 and cases.relerr(fb, st["b_adv"]) < 1e-12, sstep
-        assert np.abs(fr - g["r_fs"][k]).max() < 1e-12 and np.abs(fb - g["b_fs"][k]).max() < 1e-12, sstep
+        rows = g["rows"]  # the reference driver's fields are stored on every 10th row
+        assert np.abs(fr[rows] - g["r_fs"][k]).max() < 1e-12 and np.abs(fb[rows] - g["b_fs"][k]).max() < 1e-12, sstep
         rho, u = d.get_moments()
-        assert np.abs(rho[..., 0] - g["rho"][k]).max() < 1e-12, sstep
-        assert np.abs(u[..., 0] - g["ux"][k]).max() < 1e-12 and np.abs(u[..., 1] - g["uy"][k]).max() < 1e-12, sstep
+        assert np.abs(rho[rows, :, 0] - g["rho"][k]).max() < 1e-12, sstep
+        assert np.abs(u[rows, :, 0] - g["ux"][k]).max() < 1e-12 and np.abs(u[rows, :, 1] - g["uy"][k]).max() < 1e-12, sstep
 
 
 def test_rk_long_run_stays_on_the_oracle(orc):
@@ -265,7 +266,7 @@ def test_rk_diagnostic_fields_vs_oracle_and_golden(orc):
             assert np.abs(got[k] - want[k]).max() < 1e-12 * max(scale[k], 1e-3), (n, k)
         if n in steps:
             for name, a in rk_diag_fields(got).items():
-                assert np.abs(a - g[name][steps.index(n)]).max() < 1e-12, (n, name)
+                assert np.abs(a[g["rows"]] - g[name][steps.index(n)]).max() < 1e-12, (n, name)
         orc.rk_step(p, st)
         d.step(1)
     assert cases.relerr(d.get_f(0), st["r_adv"]) < 1e-12  # asking for diagnostics between steps does not disturb the state
@@ -303,5 +304,5 @@ def test_rk_driver_writes_all_nineteen_reference_files(tmp_path):
         if key is not None:
             for k, s in enumerate(int(s) for s in g["steps"]):
                 if s < 12:
-                    assert np.abs(a[..., s] - g[key][k]).max() < 1e-12, (fname, s)
+                    assert np.abs(a[g["rows"]][..., s] - g[key][k]).max() < 1e-12, (fname, s)
     assert np.abs(got["omegas3"] - (got["omegas1"] + got["omegas2"])).max() < 1e-15

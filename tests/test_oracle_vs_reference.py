@@ -1,6 +1,11 @@
-"""CPU, only where oracle/_ref exists (this container): the oracle and the product's host-side
-parameter code against the unmodified reference library through oracle/ref_harness.cpp."""
+"""CPU: the oracle and the product's host-side parameter code against the unmodified reference library.
+
+Where the fixtures under tests/golden hold what the reference computed (make_golden.py stored it from oracle/_ref), the
+comparison runs everywhere against them; where oracle/_ref is built (make -C oracle ref REF=<checkout of the original
+sources>, or build() with LBM_REFERENCE_DIR set) the same tests also compare live through oracle/ref_harness.cpp, and the
+tests without stored outputs run only there."""
 import os
+import tomllib
 
 import numpy as np
 import pytest
@@ -9,7 +14,7 @@ import cases
 import lbm_b200 as L
 from oracle_lib import Oracle, Ref, have_ref
 
-pytestmark = [pytest.mark.ref, pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built (needs /root/reference)")]
+needs_ref = pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built (needs the original sources)")
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PARAMS = os.path.join(ROOT, "configs", "parameters.toml")
@@ -21,6 +26,8 @@ def libs():
     return Oracle(), Ref()
 
 
+@pytest.mark.ref
+@needs_ref
 def test_granular_ops(libs):
     o, r = libs
     rng = np.random.default_rng(0)
@@ -40,6 +47,8 @@ def test_granular_ops(libs):
             assert np.array_equal(o.advect(f), r.advect(f))
 
 
+@pytest.mark.ref
+@needs_ref
 def test_differential_incl_replicate_padding(libs):
     o, r = libs
     rng = np.random.default_rng(1)
@@ -55,9 +64,24 @@ def test_differential_incl_replicate_padding(libs):
     assert np.abs(dy[:, 2:-2] - 1.0).max() < 1e-13 and np.abs(dx).max() < 1e-13
 
 
-def test_params_bit_exact(libs):
-    o, r = libs
-    ref = r.params(PARAMS, True)
+def test_params_bit_exact(tmp_path):
+    """params::lattice of the product against the reference's: omega, u and the grid the reference derived from the TOML
+    files of three fixtures (make_golden.py stored them), and with oracle/_ref every field for configs/parameters.toml"""
+    o = Oracle()
+    for name in ("free_stream_33x22", "cylinder_99x77", "sedimentation_176x264"):
+        g = cases.golden(name)
+        path = tmp_path / f"{name}.toml"
+        path.write_text(str(g["toml"]))
+        mine = L.params_from_toml(str(path), True)
+        assert (mine.X, mine.Y) == (int(g["X"]), int(g["Y"])) and mine.omega == float(g["omega"]), name
+        assert "u_lb" not in g or mine.u == float(g["u_lb"]), name
+        la = tomllib.loads(str(g["toml"]))["lattice"]
+        op = o.params_lattice(mine.flow_rho_0, mine.flow_nu, mine.flow_u, mine.flow_l, mine.tau, mine.dx, la["x_multiplier"],
+                              la["y_multiplier"])
+        assert (op["X"], op["Y"]) == (mine.X, mine.Y) and op["omega"] == mine.omega and op["u"] == mine.u, name
+    if not have_ref():
+        return
+    ref = Ref().params(PARAMS, True)
     mine = L.params_from_toml(PARAMS, True)
     for k_ref, k in [("fp_nu", "flow_nu"), ("fp_u", "flow_u"), ("fp_l", "flow_l"), ("fp_rho_0", "flow_rho_0"),
                      ("fp_Re", "flow_Re"), ("tau", "tau"), ("omega", "omega"), ("Re", "Re"), ("nu", "nu"), ("l", "l"),
@@ -71,6 +95,8 @@ def test_params_bit_exact(libs):
     assert op["u"] == mine.u and op["dt"] == mine.dt and op["omega"] == mine.omega
 
 
+@pytest.mark.ref
+@needs_ref
 def test_colour_bit_exact(libs):
     o, r = libs
     for table in ("red", "blue"):
@@ -84,13 +110,30 @@ def test_colour_bit_exact(libs):
         assert np.array_equal(oc["eta"], ref["eta"])
 
 
+@pytest.mark.ref
+@needs_ref
 def test_domain_shapes(libs):
     _, r = libs
     assert r.domain_shapes(21, 33) == [(21, 33, 9)] * 3 + [(21, 33, 1), (21, 33, 2)]
 
 
-def test_ibm_force(libs, tmp_path):
-    o, r = libs
+def test_ibm_force(tmp_path):
+    """the reference's ibm class on a seeded field around the cylinder fixture's markers (make_golden.py stored its
+    force), and with oracle/_ref live on a second body"""
+    o = Oracle()
+    g = cases.golden("cylinder_99x77")
+    path = tmp_path / "cylinder.toml"
+    path.write_text("[cylinder-a]\nx = [" + ", ".join(repr(float(v)) for v in g["marker_x"]) + "]\ny = [" +
+                    ", ".join(repr(float(v)) for v in g["marker_y"]) + "]\n")
+    mx, my = L.markers_from_toml(str(path), "cylinder-a")
+    assert np.array_equal(mx, g["marker_x"]) and np.array_equal(my, g["marker_y"])
+    ib = o.ibm_create(mx, my)
+    assert o.ibm_roi(ib) == tuple(int(v) for v in g["roi"])
+    assert cases.relerr(o.ibm_force(ib, g["ibm_u"], g["ibm_rho"]), g["ibm_F"]) < 1e-14
+    o.ibm_destroy(ib)
+    if not have_ref():
+        return
+    r = Ref()
     th = 2 * np.pi * np.arange(57) / 57
     xs, ys = 20.3 + 7.7 * np.cos(th), 17.9 + 6.1 * np.sin(th)
     path = tmp_path / "b.toml"
@@ -108,6 +151,8 @@ def test_ibm_force(libs, tmp_path):
     o.ibm_destroy(ib)
 
 
+@pytest.mark.ref
+@needs_ref
 def test_kbc_class_and_driver_loops(libs):
     """ulbm::d2q9::kbc (src/ulbm.cpp) through ref_kbc_run: both drivers' loop bodies, warm and cold starts"""
     o, r = libs
@@ -134,13 +179,24 @@ def test_kbc_class_and_driver_loops(libs):
         assert np.abs(fo - fr).max() < 1e-12, n
 
 
-def test_poiseuille_loop_of_the_reference_matches_the_port(libs):
-    """the timed loop bench.py uses as the CPU arm of the poiseuille workload (oracle/ref_harness.cpp: the reference's own
-    operators in the order of test/horizontal_poiseuille_test.cpp:100-153) lands where the C port's step does"""
-    orc, ref = libs
-    H, W, steps = 21, 21, 60
+def test_poiseuille_loop_of_the_reference_matches_the_port():
+    """the C port's step lands where the reference's Poiseuille loop does: the checksum of the populations after 100 steps of
+    the reference driver (the poiseuille fixture), and with oracle/_ref after 60 steps of the timed loop bench.py uses as the
+    CPU arm of the poiseuille workload (oracle/ref_harness.cpp: the reference's own operators in the order of
+    test/horizontal_poiseuille_test.cpp:100-153)"""
+    orc = Oracle()
+    H, W = 21, 21
     omega, rho_in, rho_out = cases.channel_constants(H, W, 1.030985714e-1)
-    _, chk = ref.poiseuille_loop(H, W, omega, rho_in, rho_out, 0, steps)
+    g = cases.golden("poiseuille_21x21")
+    k = [int(s) for s in g["steps"]].index(100)
+    f = g["f"][0].copy(); u = np.zeros((H, W, 2)); rho = np.ones((H, W, 1))
+    for _ in range(100):
+        orc.poiseuille_step(f, u, rho, omega, rho_in, rho_out)
+    assert abs(g["f"][k].sum() - f.sum()) < 1e-11 * abs(f.sum())
+    if not have_ref():
+        return
+    steps = 60
+    _, chk = Ref().poiseuille_loop(H, W, omega, rho_in, rho_out, 0, steps)
     u = np.zeros((H, W, 2)); rho = np.ones((H, W, 1))
     f = orc.incomp_equilibrium(u, rho)
     for _ in range(steps):
