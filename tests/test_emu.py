@@ -54,14 +54,16 @@ def test_gpu_parity_tests_pass_on_the_emulated_device(emu_lib):
 @pytest.mark.parametrize("order", ["reverse", "shuffle:3"])
 def test_shared_memory_ring_kernels_do_not_depend_on_thread_order(emu_lib, order):
     """The threads of a block start and resume in reversed / shuffled order.  A missing barrier around the shared-memory
-    rings of k_tp_fused / k_csf_collide_ring makes these runs fail (checked by deleting the ring's __syncthreads)."""
-    r = run_emulated(["tests/test_gpu_two_phase.py", "tests/test_gpu_csf.py"], 900, order)
+    rings of k_tp_fused / k_csf_collide_ring makes these runs fail (checked by deleting the ring's __syncthreads).  Every
+    instantiation of the two-phase step runs here too (test_gpu_tp_variants.py: stage slots, mbarrier parities, ring rows)."""
+    r = run_emulated(["tests/test_gpu_two_phase.py", "tests/test_gpu_csf.py", "tests/test_gpu_tp_variants.py"], 900, order)
     assert r.returncode == 0, r.stdout[-4000:]
 
 
 def test_kernels_under_address_sanitizer():
     """Device buffers are heap blocks of the emulated runtime: an out-of-bounds load or store of a kernel (or of the host
-    code around it) is an AddressSanitizer report.  The two-phase and CSF tests here (ragged and tiny grids included); `make -C tests/cpu_emu SAN=1` + LBM_EMU_ASAN=1 runs any of the others the same way."""
+    code around it) is an AddressSanitizer report.  The two-phase and CSF tests here (ragged and tiny grids included, every
+    two-phase kernel instantiation at one-row bands); `make -C tests/cpu_emu SAN=1` + LBM_EMU_ASAN=1 runs any of the others the same way."""
     asan = subprocess.run(["/usr/bin/gcc", "-print-file-name=libasan.so"], capture_output=True, text=True).stdout.strip()
     if not os.path.isabs(asan) or not os.path.exists(asan):
         pytest.skip("no libasan next to the system gcc")
@@ -70,7 +72,7 @@ def test_kernels_under_address_sanitizer():
     env = dict(os.environ, LBM_EMU="1", LBM_EMU_ASAN="1", OMP_WAIT_POLICY="passive", LD_PRELOAD=asan,
                ASAN_OPTIONS="detect_leaks=0:abort_on_error=1:verify_asan_link_order=0")
     cmd = [sys.executable, "-m", "pytest", "-m", "gpu", "-q", "-x", "-p", "no:cacheprovider",
-           "tests/test_gpu_two_phase.py", "tests/test_gpu_csf.py"]
+           "tests/test_gpu_two_phase.py", "tests/test_gpu_csf.py", "tests/test_gpu_tp_variants.py"]
     r = subprocess.run(cmd, cwd=ROOT, env=env, capture_output=True, text=True, timeout=1500)
     assert r.returncode == 0 and "AddressSanitizer" not in r.stdout + r.stderr, r.stdout[-3000:] + r.stderr[-3000:]
 

@@ -18,17 +18,36 @@ BUDGET = {
     "k_bgk_interiorILi1ELi1ELi0ELb0E": (80, "BGK pull, incompressible (Poiseuille)"),
     "k_bgk_interiorILi1ELi0ELi0ELb1E": (100, "BGK + advection-diffusion lattice (sedimentation)"),
     "k_bgk_interiorILi1ELi2ELi0ELb0E": (128, "KBC: 4 resident blocks of 128 threads"),
-    "k_tp_stagedILi0ELi3ELi3ELb1E": (168, "MRT colour gradient, staged rows + tensor-memory stash (the default): 3 resident blocks"),
-    "k_tp_stagedILi1ELi4ELi2ELb1E": (168, "Rothman-Keller, staged rows + tensor-memory stash (the default): 2 resident blocks by shared memory"),
-    "k_tp_stagedILi0ELi5ELi2ELb0E": (255, "MRT colour gradient, rows resident in the stage slots (LBM_TP_STASH=0): 2 resident blocks"),
+    # the two-phase step: every instantiation tp_launch_fused can launch (tests/test_gpu_tp_variants.py runs each of them)
+    "k_tp_stagedILi0ELi3ELi3ELb1E": (168, "MRT colour gradient, staged rows + tensor-memory stash, NS = 3 (the default): 3 resident blocks"),
+    "k_tp_stagedILi0ELi2ELi4ELb1E": (128, "MRT colour gradient, staged rows + tensor-memory stash, NS = 2: 4 resident blocks"),
+    "k_tp_stagedILi0ELi4ELi2ELb1E": (168, "MRT colour gradient, staged rows + tensor-memory stash, NS = 4: 2 resident blocks"),
+    "k_tp_stagedILi0ELi4ELi2ELb0E": (168, "MRT colour gradient, rows resident in the stage slots, NS = 4: 2 resident blocks"),
+    "k_tp_stagedILi0ELi5ELi2ELb0E": (168, "MRT colour gradient, rows resident in the stage slots, NS = 5 (LBM_TP_STASH=0): 2 resident blocks"),
+    "k_tp_stagedILi0ELi6ELi2ELb0E": (168, "MRT colour gradient, rows resident in the stage slots, NS = 6: 2 resident blocks"),
+    "k_tp_stagedILi1ELi5ELi2ELb0E": (168, "Rothman-Keller, rows resident in the stage slots, NS = 5 (the default): 2 resident blocks"),
+    "k_tp_stagedILi1ELi3ELi3ELb0E": (168, "Rothman-Keller, rows resident in the stage slots, NS = 3: 3 resident blocks"),
+    "k_tp_stagedILi1ELi4ELi2ELb0E": (168, "Rothman-Keller, rows resident in the stage slots, NS = 4: 2 resident blocks"),
+    "k_tp_stagedILi1ELi6ELi2ELb0E": (168, "Rothman-Keller, rows resident in the stage slots, NS = 6: 2 resident blocks"),
+    "k_tp_stagedILi1ELi2ELi4ELb1E": (128, "Rothman-Keller, staged rows + tensor-memory stash, NS = 2: 4 resident blocks"),
+    "k_tp_stagedILi1ELi3ELi3ELb1E": (168, "Rothman-Keller, staged rows + tensor-memory stash, NS = 3: 3 resident blocks"),
+    "k_tp_stagedILi1ELi4ELi2ELb1E": (168, "Rothman-Keller, staged rows + tensor-memory stash, NS = 4 (LBM_TP_STASH=1): 2 resident blocks by shared memory"),
     "k_csf_stagedILi3ELb1E": (208, "CSF single pass, staged rows + tensor-memory stash (the default): 2 resident blocks"),
     "k_tp_fusedILi0ELb1E": (168, "MRT colour gradient, pipelined: 3 resident blocks"),
+    "k_tp_fusedILi0ELb0E": (128, "MRT colour gradient, plain (LBM_TP_PIPE=0): 4 resident blocks"),
     "k_tp_fusedILi1ELb1E": (168, "Rothman-Keller, pipelined: 3 resident blocks"),
+    "k_tp_fusedILi1ELb0E": (168, "Rothman-Keller, plain (LBM_TP_PIPE=0): 3 resident blocks"),
     "k_csf_collide_ringILi1E": (168, "CSF collision pass: 3 resident blocks"),
     "k_csf_fusedILb0E": (168, "CSF single pass, plain: 3 resident blocks"),
     "k_csf_fusedILb1E": (255, "CSF single pass, pipelined: 2 resident blocks"),
     "k_bgk_interiorILi1ELi0ELi2ELb1E": (110, "BGK + advection-diffusion lattice + IBM force field (sedimentation_ibm)"),
 }
+
+# mangled-name fragment -> stack frame (bytes) allowed.  k_tp_fused<MRTCG, false> is held to 128 registers by its launch
+# bounds (four resident blocks) and spills three words into a 16-byte frame (ptxas: 12 bytes of spill stores and loads); it is
+# a non-default instantiation (LBM_TP_STAGED=0 LBM_TP_PIPE=0) kept as the plain reference of the others, so the spill is
+# recorded here rather than traded for its occupancy.  Every other kernel listed above spills nothing.
+SPILL_ALLOWED = {"k_tp_fusedILi0ELb0E": 16}
 
 
 @pytest.mark.skipif(shutil.which("cuobjdump") is None, reason="cuobjdump not on PATH")
@@ -51,4 +70,4 @@ def test_step_kernels_stay_within_their_register_budget():
         assert frag in found, f"{what}: kernel {frag} not found in the library"
         reg, stack, local = found[frag]
         assert reg <= limit, f"{what}: {reg} registers > {limit}"
-        assert stack == 0 and local == 0, f"{what}: spills (stack {stack}, local {local})"
+        assert stack <= SPILL_ALLOWED.get(frag, 0) and local == 0, f"{what}: spills (stack {stack}, local {local})"
