@@ -275,6 +275,29 @@ int lbm_ibm_get_force(lbm_domain* d, double* F_aos);
 int lbm_ibm_force(lbm_domain* d, const double* u_aos, const double* rho_aos, double* F_aos);
 
 /* ------------------------------------------------------------------------------------------------
+ * Force on a body, recorded on the device every step — replaces the accumulation of F_s that test/cylinder_test.cpp:112
+ * snapshots for an offline sum.  Each domain records the force that the fluid on ITS rows exerts on one body, in lattice
+ * units, for the step that advances f_coll(t) to f_adve(t+1); the parts of linked slabs / ring ranks add up to the total.
+ *   bounce-back body: momentum exchange F = sum 2 c_opp(q) f_coll(t)[n, opp(q)] over the links (n, q) with n a fluid node
+ *                     of this slab and n - c_q solid (periodic wrap, as lbm_bc_add_solid)
+ *   immersed body:    F = -sum F_euler over the ROI nodes of this slab's rows (F_euler: the field the step adds)
+ * The sum is deterministic (no floating-point atomics) and lands in a device ring; nothing crosses to the host until
+ * lbm_body_force_read.  Single-phase models only (two-phase: LBM_ERR_UNSUPPORTED).  Without a record the step is unchanged.
+ * ---------------------------------------------------------------------------------------------- */
+/* solid != NULL: the staircase body of lbm_bc_add_solid(d, 0, solid, X, Y) ({X,Y} GLOBAL mask); needs lbm_bc_commit first,
+ *                and every counted link must be owned by a plain bounce-back LBM_BC_LINEAR op (same node, src_q = opp(q),
+ *                coef 1, cst 0), else LBM_ERR_INVALID.  A later lbm_bc_commit / lbm_bc_clear ends the record.
+ * solid == NULL: the immersed body of lbm_ibm_set_markers (F_s of test/cylinder_test.cpp:112, sign flipped); X, Y are
+ *                ignored.  A later lbm_ibm_set_markers / lbm_set_force_region ends the record.
+ * capacity = steps kept in the device ring.  Calling it again replaces the record and restarts the count. */
+int lbm_body_force_record(lbm_domain* d, const unsigned char* solid, int X, int Y, int capacity);
+/* Force on the body from the last min(recorded, capacity, max_steps) steps, in step order.
+ * F[2k] is along axis 0 (x, rows) and F[2k+1] along axis 1.  *first_step is the index of entry 0,
+ * counted from the record call.  Synchronises the domain's stream. */
+int lbm_body_force_read(lbm_domain* d, double* F, int max_steps, int* n_steps, long long* first_step);
+int lbm_body_force_stop(lbm_domain* d);
+
+/* ------------------------------------------------------------------------------------------------
  * Time stepping — replaces the loop body of each driver (SURVEY §3.1-3.3)
  * ---------------------------------------------------------------------------------------------- */
 /* advance n_steps; asynchronous on the domain's stream */

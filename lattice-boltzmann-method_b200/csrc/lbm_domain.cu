@@ -397,6 +397,7 @@ int step_side_tail(lbm_domain* d, bool exchange_local, bool with_ibm)
     ProfScope ps(d, LBM_PROF_IBM, d->side);
     LBM_TRY(ibm_prepass(d, MODE_PULL, t, d->ibm.next_slot ^ 1, d->side));
   }
+  LBM_TRY(body_force_step(d));
   LBM_CUDA(cudaEventRecord(d->ev_side, d->side));
   return LBM_OK;
 }
@@ -565,6 +566,7 @@ void drop_graphs(lbm_domain* d)
 static void release_compiled(lbm_domain* d)
 {
   drop_graphs(d);
+  if (d->bf.on && !d->bf.immersed) body_force_release(d);  // its links were checked against the rules being replaced
   cudaFree(d->d_bx); cudaFree(d->d_by); cudaFree(d->d_ent); cudaFree(d->d_mom[0]); cudaFree(d->d_mom[1]);
   d->d_bx = d->d_by = nullptr; d->d_ent = nullptr; d->d_mom[0] = d->d_mom[1] = nullptr;
   for (auto& sg : d->stages)
@@ -1492,3 +1494,6 @@ int lbm_decompose_rows(int X, int n_ranks, int rank, int* x0, int* x1)
 }
 
 }  // extern "C"
+
+// lbm_body_force_record / _read / _stop and their kernels
+#include "lbm_body_force.cuh"

@@ -120,6 +120,7 @@ __global__ void k_ibm_pack_force(int nn, const double* __restrict__ Fx, const do
 int ibm_release(lbm_domain* d)
 {
   IbmState& ib = d->ibm;
+  if (d->bf.on && d->bf.immersed) body_force_release(d);  // it reads the active list and force fields freed here
   cudaFree(ib.d_active); cudaFree(ib.d_mrow); cudaFree(ib.d_mcol); cudaFree(ib.d_phi); cudaFree(ib.d_fj); cudaFree(ib.d_ptr);
   cudaFree(ib.d_ent_marker); cudaFree(ib.d_ent_phi); cudaFree(ib.d_u); cudaFree(ib.d_rho);
   for (int k = 0; k < 2; k++) { cudaFree(ib.d_Fx[k]); cudaFree(ib.d_Fy[k]); }

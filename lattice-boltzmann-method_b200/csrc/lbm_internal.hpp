@@ -97,6 +97,19 @@ struct IbmGiven
   unsigned long long hash = 0;
 };
 
+// lbm_body_force_record: the force on one body, summed on the device once per step into a ring (lbm_body_force.cuh)
+struct BodyForce
+{
+  bool on = false;
+  bool immersed = false;          // the immersed body's force field; otherwise the bounce-back links of a solid mask
+  int capacity = 0;               // steps the ring keeps
+  int n = 0;                      // links, or active ROI nodes on this slab's rows
+  long long* d_link = nullptr;    // [n] (offset of f[opp(q)] at the link's fluid node in a lattice buffer) << 4 | q, by (node, q)
+  double* d_part = nullptr;       // [blocks][2] per-block partial sums
+  double* d_ring = nullptr;       // [capacity][2]
+  long long* d_count = nullptr;   // steps recorded so far (advanced by the kernel, so graph replays count too)
+};
+
 struct ProfRec
 {
   cudaEvent_t a, b;
@@ -198,6 +211,7 @@ struct lbm_domain
 
   lbm::IbmState ibm;
   lbm::IbmGiven ibm_given;
+  lbm::BodyForce bf;
   double ics2 = 1.0 / 3.0, ics4 = 1.0 / 9.0;  // source-term constants (lbm_set_force_region overrides them)
   // column-face bindings to other blocks (lbm_link_face): the populations entering through an edge column are read
   // from a tail appended to every lattice buffer, [side][3 populations][Xl] behind the nine planes
@@ -254,6 +268,9 @@ int ibm_roi_local(lbm_domain* d, int mode, int which, cudaStream_t st);  // mome
 int ibm_iterate(lbm_domain* d, int slot, cudaStream_t st);               // forcing iterations on the complete ROI fields
 int comm_ibm_share(lbm_domain* d, cudaStream_t st);
 int faces_release(lbm_domain* d);                      // NCCL: ROI row segments between the slabs that own ROI rows
+// lbm_body_force.cuh (compiled inside lbm_domain.cu)
+void body_force_release(lbm_domain* d);
+int body_force_step(lbm_domain* d);  // side: the force of the step being enqueued into the ring (no-op when not recording)
 // lbm_two_phase.cu
 int tp_create(lbm_domain* d);
 int tp_destroy(lbm_domain* d);

@@ -106,6 +106,7 @@ EXPORTS = [
     "lbm_preset_sedimentation", "lbm_preset_mrtcg", "lbm_preset_rk", "lbm_preset_periodic",
     "lbm_profile_enable", "lbm_profile_read", "lbm_step_group", "lbm_save_pt", "lbm_snapshot_async", "lbm_snapshot_wait", "lbm_set_moments", "lbm_get_interfacial_tension", "lbm_link_face", "lbm_set_force_region",
     "lbm_rk_diagnostics", "lbm_comm_check", "lbm_comm_share", "lbm_row_split", "lbm_comm_init_blocks", "lbm_link_face_rank", "lbm_comm_faces_commit",
+    "lbm_body_force_record", "lbm_body_force_read", "lbm_body_force_stop",
 ]
 PROF_INTERIOR, PROF_BOUNDARY, PROF_FIXUP, PROF_GHOST, PROF_IBM, PROF_MOMENTS, PROF_EARLY = range(7)
 
@@ -147,6 +148,9 @@ def load():
         _lib.lbm_ibm_get_roi.argtypes = [C.c_void_p, C.POINTER(C.c_long)]
         _lib.lbm_ibm_get_force.argtypes = [C.c_void_p, dp]
         _lib.lbm_ibm_force.argtypes = [C.c_void_p, dp, dp, dp]
+        _lib.lbm_body_force_record.argtypes = [C.c_void_p, C.POINTER(C.c_ubyte), C.c_int, C.c_int, C.c_int]
+        _lib.lbm_body_force_read.argtypes = [C.c_void_p, dp, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_longlong)]
+        _lib.lbm_body_force_stop.argtypes = [C.c_void_p]
         _lib.lbm_step.argtypes = [C.c_void_p, C.c_int]
         _lib.lbm_last_step_ms.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
         _lib.lbm_kernel_launches.argtypes = [C.c_void_p, C.POINTER(C.c_longlong)]
@@ -400,6 +404,34 @@ class Domain:
         _chk(self.lib.lbm_ibm_force(self.h, ap, bp, F.ctypes.data_as(dp)))
         return F
 
+    # ---- force on a body, recorded on the device every step
+    def body_force_record(self, solid=None, capacity=4096):
+        """record the force on the bounce-back body of the GLOBAL {X,Y} mask `solid` (as given to bc_add_solid, after
+        bc_commit), or with solid=None on the immersed body of ibm_set_markers; the last `capacity` steps are kept"""
+        if solid is None:
+            _chk(self.lib.lbm_body_force_record(self.h, None, self.cfg.X, self.cfg.Y, int(capacity)))
+        else:
+            m = np.ascontiguousarray(solid, dtype=np.uint8)
+            if m.shape != (self.cfg.X, self.cfg.Y):
+                raise ValueError("solid mask must have the global shape {X,Y}")
+            _chk(self.lib.lbm_body_force_record(self.h, m.ctypes.data_as(C.POINTER(C.c_ubyte)), m.shape[0], m.shape[1],
+                                                int(capacity)))
+        self._bf_capacity = int(capacity)
+
+    def body_force(self, max_steps=None):
+        """(F, first_step): F {n,2} float64, the force on the body (axis 0, axis 1) of the last n recorded steps in step
+        order, first_step the index of F[0] counted from body_force_record.  Synchronises the domain."""
+        cap = getattr(self, "_bf_capacity", 0)
+        m = cap if max_steps is None else int(max_steps)
+        F = np.empty((max(m, 1), 2))
+        n = C.c_int(); first = C.c_longlong()
+        _chk(self.lib.lbm_body_force_read(self.h, F.ctypes.data_as(dp), m, C.byref(n), C.byref(first)))
+        return F[:n.value].copy(), first.value
+
+    def body_force_stop(self):
+        _chk(self.lib.lbm_body_force_stop(self.h))
+        self._bf_capacity = 0
+
     # ---- stepping
     def step(self, n=1):
         _chk(self.lib.lbm_step(self.h, int(n)))
@@ -473,6 +505,17 @@ def step_group(domains, n_steps=1):
     """advance linked slabs in lock step"""
     arr = (C.c_void_p * len(domains))(*[d.h for d in domains])
     _chk(load().lbm_step_group(arr, len(domains), int(n_steps)))
+
+
+def body_force_group(domains, max_steps=None):
+    """(F, first_step) of one body over linked slabs: the sum of every slab's part (each records the fluid on its rows)"""
+    parts = [d.body_force(max_steps) for d in domains]
+    if any(p[1] != parts[0][1] or len(p[0]) != len(parts[0][0]) for p in parts):
+        raise ValueError("body_force_group: the slabs' records cover different steps (record on every slab, then step them together)")
+    F = parts[0][0].copy()
+    for p in parts[1:]:
+        F += p[0]
+    return F, parts[0][1]
 
 
 def comm_unique_id():
