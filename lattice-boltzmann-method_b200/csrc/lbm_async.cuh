@@ -19,10 +19,6 @@ namespace lbm
 
 #if !defined(LBM_CPU_EMU)
 
-#ifndef LBM_TMEM_X4
-#define LBM_TMEM_X4 0
-#endif
-
 __device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 __device__ __forceinline__ void mbar_init(uint64_t* bar, unsigned count)
@@ -104,11 +100,6 @@ __device__ __forceinline__ void tmem_store18(uint32_t taddr, const double (&a)[9
     r[18 + 2 * q] = (uint32_t)__double2loint(b[q]);
     r[18 + 2 * q + 1] = (uint32_t)__double2hiint(b[q]);
   }
-#if LBM_TMEM_X4  // experiment switch: nine 4-column accesses instead of 32 + 4 columns
-#pragma unroll
-  for (int c = 0; c < 36; c += 4)
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(taddr + (unsigned)c), "r"(r[c]), "r"(r[c + 1]), "r"(r[c + 2]), "r"(r[c + 3]) : "memory");
-#else
   asm volatile(
       "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, %17, %18, %19, %20, "
       "%21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};" ::"r"(taddr),
@@ -118,7 +109,6 @@ __device__ __forceinline__ void tmem_store18(uint32_t taddr, const double (&a)[9
       : "memory");
   asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(taddr + 32u), "r"(r[32]), "r"(r[33]), "r"(r[34]), "r"(r[35])
                : "memory");
-#endif
 }
 
 __device__ __forceinline__ void tmem_store_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
@@ -127,11 +117,6 @@ __device__ __forceinline__ void tmem_store_wait() { asm volatile("tcgen05.wait::
 // asynchronously), later wait, then read the registers
 __device__ __forceinline__ void tmem_load18_issue(uint32_t taddr, uint32_t (&r)[36])
 {
-#if LBM_TMEM_X4
-#pragma unroll
-  for (int c = 0; c < 36; c += 4)
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(r[c]), "=r"(r[c + 1]), "=r"(r[c + 2]), "=r"(r[c + 3]) : "r"(taddr + (unsigned)c) : "memory");
-#else
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, %17, %18, %19, %20, "
       "%21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
@@ -142,7 +127,6 @@ __device__ __forceinline__ void tmem_load18_issue(uint32_t taddr, uint32_t (&r)[
       : "r"(taddr)
       : "memory");
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(r[32]), "=r"(r[33]), "=r"(r[34]), "=r"(r[35]) : "r"(taddr + 32u) : "memory");
-#endif
 }
 __device__ __forceinline__ void tmem_load_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_unpack18(uint32_t (&r)[36], double (&a)[9], double (&b)[9])

@@ -836,7 +836,7 @@ static int group_faces(lbm_domain* const* ds, int n, bool new_buffer)
       for (int j = 0; j < n; j++) member = member || ds[j] == o;
       if (!member || !o->have_state) { set_error("lbm_step_group: a block is bound to a block outside the group"); return LBM_ERR_INVALID; }
       const int ow = new_buffer ? o->cur ^ 1 : o->cur, dw = new_buffer ? d->cur ^ 1 : d->cur;
-      LBM_CUDA(cudaSetDevice(o->cfg.device));
+      LBM_CUDA(on(o));
       LBM_CUDA(cudaStreamWaitEvent(o->side, d->ev_side, 0));  // the copy out of this packet one step ago
       const int total = d->nlat * 3 * fl.n;
       k_face_pack<<<(total + 127) / 128, 128, 0, o->side>>>(o->buf[0][ow], o->buf[1][ow], o->g, fl.side == 0 ? o->g.Y - 1 : 0, fl.orb,
@@ -844,7 +844,7 @@ static int group_faces(lbm_domain* const* ds, int n, bool new_buffer)
       o->launches++;
       LBM_CUDA(cudaGetLastError());
       LBM_CUDA(cudaEventRecord(fl.ev, o->side));
-      LBM_CUDA(cudaSetDevice(d->cfg.device));
+      LBM_CUDA(on(d));
       LBM_CUDA(cudaStreamWaitEvent(d->side, fl.ev, 0));
       ProfScope ps(d, LBM_PROF_GHOST, d->side);
       for (int l = 0; l < d->nlat; l++)
@@ -862,16 +862,14 @@ static int group_faces(lbm_domain* const* ds, int n, bool new_buffer)
 // enqueued (side tail) rather than to this one (prologue).
 static int group_ibm(lbm_domain* const* ds, int n, bool tail)
 {
-  auto uses = [](const lbm_domain* d) { return d->ibm.enabled && !d->ibm.fixed && d->cfg.force == LBM_FORCE_IBM; };
-  auto on = [](lbm_domain* d) { return cudaSetDevice(d->cfg.device); };
   for (int i = 0; i < n; i++)
   {
     lbm_domain* d = ds[i];
-    if (!uses(d) || (!tail && d->side_ready)) continue;
+    if (!uses_ibm(d) || (!tail && d->side_ready)) continue;
     LBM_CUDA(on(d));
     if (d->ibm.split)  // the other owners may still be copying the segment of the pre-pass before
       for (int j = 0; j < n; j++)
-        if (j != i && uses(ds[j]) && ds[j]->ibm.split) LBM_CUDA(cudaStreamWaitEvent(d->side, ds[j]->ev_side, 0));
+        if (j != i && uses_ibm(ds[j]) && ds[j]->ibm.split) LBM_CUDA(cudaStreamWaitEvent(d->side, ds[j]->ev_side, 0));
     ProfScope ps(d, LBM_PROF_IBM, d->side);
     const int mode = tail ? MODE_PULL : (d->post_stream ? MODE_LOCAL : MODE_PULL);
     LBM_TRY(ibm_roi_local(d, mode, tail ? d->cur ^ 1 : d->cur, d->side));
@@ -880,7 +878,7 @@ static int group_ibm(lbm_domain* const* ds, int n, bool tail)
   for (int i = 0; i < n; i++)
   {
     lbm_domain* d = ds[i];
-    if (!uses(d) || (!tail && d->side_ready)) continue;
+    if (!uses_ibm(d) || (!tail && d->side_ready)) continue;
     LBM_CUDA(on(d));
     ProfScope ps(d, LBM_PROF_IBM, d->side);
     if (d->ibm.split)
@@ -889,7 +887,7 @@ static int group_ibm(lbm_domain* const* ds, int n, bool tail)
       for (int j = 0; j < n; j++)
       {
         lbm_domain* o = ds[j];
-        if (j == i || !uses(o) || o->ibm.row_hi <= o->ibm.row_lo) continue;
+        if (j == i || !uses_ibm(o) || o->ibm.row_hi <= o->ibm.row_lo) continue;
         if (o->ibm.r0 != d->ibm.r0 || o->ibm.r1 != d->ibm.r1 || o->ibm.n_markers != d->ibm.n_markers)
         {
           set_error("lbm_step_group: slabs %d and %d carry different immersed bodies (hand every slab the same marker list)", i, j);
@@ -907,12 +905,12 @@ static int group_ibm(lbm_domain* const* ds, int n, bool tail)
   for (int i = 0; i < n; i++)
   {
     lbm_domain* d = ds[i];
-    if (!uses(d) || (!tail && d->side_ready)) continue;
+    if (!uses_ibm(d) || (!tail && d->side_ready)) continue;
     LBM_CUDA(on(d));
     ProfScope ps(d, LBM_PROF_IBM, d->side);
     if (d->ibm.split)
       for (int j = 0; j < n; j++)
-        if (j != i && uses(ds[j]) && ds[j]->ibm.split) LBM_CUDA(cudaStreamWaitEvent(d->side, ds[j]->ev_ibm_got, 0));
+        if (j != i && uses_ibm(ds[j]) && ds[j]->ibm.split) LBM_CUDA(cudaStreamWaitEvent(d->side, ds[j]->ev_ibm_got, 0));
     LBM_TRY(ibm_iterate(d, tail ? d->ibm.next_slot ^ 1 : d->ibm.next_slot, d->side));
     LBM_CUDA(cudaEventRecord(d->ev_side, d->side));
   }
@@ -939,7 +937,6 @@ int lbm_step_group(lbm_domain* const* ds, int n, int n_steps)
       if (!member) { set_error("lbm_step_group: block %d is bound across a column face to a block outside the group", i); return LBM_ERR_INVALID; }
     }
   if (ds[0]->tp) return tp_step_group(ds, n, n_steps);
-  auto on = [](lbm_domain* d) { return cudaSetDevice(d->cfg.device); };
   for (int i = 0; i < n; i++)
   {
     LBM_CUDA(on(ds[i]));
@@ -1013,8 +1010,7 @@ int lbm_step_group(lbm_domain* const* ds, int n, int n_steps)
     {
       lbm_domain* d = ds[i];
       LBM_CUDA(on(d));
-      for (lbm_domain* o : {d->link_lo, d->link_hi})
-        if (o && o != d) LBM_CUDA(cudaStreamWaitEvent(d->side, o->ev_stage, 0));
+      LBM_TRY(wait_linked(d, d->side, &lbm_domain::ev_stage));
       {
         ProfScope ps(d, LBM_PROF_GHOST, d->side);
         if (d->link_lo || d->link_hi) LBM_TRY(link_exchange(d, d->cur ^ 1, d->side));

@@ -260,8 +260,6 @@ int step_rows(lbm_domain* d)
   return LBM_OK;
 }
 
-static bool uses_ibm(const lbm_domain* d) { return d->ibm.enabled && !d->ibm.fixed && d->cfg.force == LBM_FORCE_IBM; }
-
 // Side chain for a state that no step has prepared (first step after an import, or an export):
 // ghost rows of buf[cur] and the IBM field the next step reads.
 int step_prologue(lbm_domain* d, bool exchange_local, bool with_ibm)

@@ -236,6 +236,17 @@ struct lbm_domain
 
 namespace lbm
 {
+// drivers of linked slabs: make the slab's device current, and let `st` wait for event `ev` of each linked neighbour
+// (a slab linked to itself waits for nothing)
+inline cudaError_t on(const lbm_domain* d) { return cudaSetDevice(d->cfg.device); }
+inline int wait_linked(const lbm_domain* d, cudaStream_t st, cudaEvent_t lbm_domain::*ev)
+{
+  for (const lbm_domain* o : {d->link_lo, d->link_hi})
+    if (o && o != d) LBM_CUDA(cudaStreamWaitEvent(st, o->*ev, 0));
+  return LBM_OK;
+}
+// the immersed body's pre-pass runs every step (markers, not a fixed region force)
+inline bool uses_ibm(const lbm_domain* d) { return d->ibm.enabled && !d->ibm.fixed && d->cfg.force == LBM_FORCE_IBM; }
 // lbm_domain.cu
 int ensure_aos_scratch(lbm_domain* d);
 void drop_graphs(lbm_domain* d);

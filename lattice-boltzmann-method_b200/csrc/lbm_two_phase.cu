@@ -22,22 +22,21 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <type_traits>
 #include <vector>
 
 #include "lbm_internal.hpp"
 #include "lbm_two_phase.cuh"
 #include "lbm_async.cuh"
 
-// L2 eviction hints of the fused kernel (see tp_pull_at); compile-time switch: 1 = the two reads, 2 = + evict_first
-// stores.  A/B on B200 (MRTCG 8192^2): DRAM reads 185 -> 165 -> 157 B/node (ideal 153), but 15.62 / 15.60 / 15.65 GLUPS
-// at 16384^2 and RK 16.84 / 16.59 / 16.27: the kernel is not DRAM-bound, the hints buy nothing.  Off by default.
-#ifndef LBM_TP_HINTS
-#define LBM_TP_HINTS 0
-#endif
-// (Also tried and dropped: prefetch.global.L2 of the next iteration's second pull, -2 %.)
+// (Tried and dropped on the fused kernel: L2 eviction-policy hints on its two reads and its stores, no gain - DESIGN §3.3;
+// prefetch.global.L2 of the next iteration's second pull, -2 %.)
 
 namespace lbm
 {
+
+struct TpKernel;   // an entry of tp_kernels / csf_kernels: the row-marching kernel of the step, chosen once per domain
+struct CsfKernel;
 
 struct TwoPhaseState
 {
@@ -53,18 +52,13 @@ struct TwoPhaseState
   int n_region = 0;
   int n_region_lo = 0, n_region_hi = 0;  // how many of them lie in rows 0, 1 (the head of the list) and Xl-2, Xl-1 (its tail)
   bool ring_overlap = false;           // LBM_TP_OVERLAP=1: the ranks of a ring send their halos behind the interior bands (tp_steps_ring)
-  int rows_per_block = 64;
-  bool pipe = true;                    // software-pipelined variant of the fused kernel (LBM_TP_PIPE=0: plain)
-  bool staged = true;                  // k_tp_staged: population rows staged by bulk async copies (LBM_TP_STAGED=0: k_tp_fused)
-  int stages = 0;                      // LBM_TP_NS: stage slots per block (0 = the model's default)
-  bool stash = true;                   // resident population rows parked in tensor memory (k_tp_staged<.., STASH>): default for MRTCG; LBM_TP_STASH=0/1
+  int rows_per_block = 64;             // band height of the row-marching kernel (band_rows, once per rule set)
+  const TpKernel* kernel = nullptr;    // TP_MRTCG / TP_RK: the row-marching kernel (LBM_TP_STAGED, LBM_TP_STASH, LBM_TP_NS, LBM_TP_PIPE)
   double* aux = nullptr;               // TP_CSF: A_COUNT planes in the moment-plane geometry (normal n, interfacial tension Fs)
   int rpb_override = 0;
-  // TP_CSF single-pass variant (LBM_CSF_FUSED=1, off by default until it has been measured on the device)
+  // TP_CSF single-pass variant
   bool csf_fused = true;               // the single-pass step (LBM_CSF_FUSED=0: three passes)
-  bool csf_pipe = false;               // LBM_CSF_PIPE=1: software-pipelined variant of k_csf_fused
-  int csf_rows = 0;                    // band height of k_csf_staged (pick_band_rows, once per rule set)
-  int csf_staged = 2;                  // single pass: 2 = k_csf_staged with the tensor-memory stash, 1 = without it, 0 = k_csf_fused
+  const CsfKernel* csf_kernel = nullptr;  // its row-marching kernel (LBM_CSF_STAGED, LBM_CSF_PIPE)
   double* aux_next = nullptr;          // second aux set: a fused step reads Fs from aux and writes it here, then the two swap
   unsigned char* d_csf_flags = nullptr;  // [Xl] bit 0: moments of the whole row from the planes; bit 1: normals too
   int* d_csf_list4 = nullptr;          // interior-column nodes whose moments the pre-pass writes to the planes
@@ -146,41 +140,10 @@ __device__ __forceinline__ void tp_load_interior(const double* __restrict__ src,
 // Pull through a per-thread node pointer (src + node_off(g, x, y)) plus WARP-UNIFORM offsets
 // q * plane - c_x * pitch - c_y: two integer instructions per access instead of a 64-bit index
 // rebuilt per thread and per population.
-// L2 eviction policies for the two reads a block makes of every line: the FIRST one (moments of row r+H) marks the
-// line evict_last so that the SECOND one (collision of the same row, LAG iterations later) still finds it in L2;
-// the second marks it evict_first.  (ncu before: only ~60 % of the second reads hit L2.)
-__device__ __forceinline__ unsigned long long l2_policy_evict_last()
-{
-  unsigned long long pol;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ unsigned long long l2_policy_evict_first()
-{
-  unsigned long long pol;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ double ld_l2_hint(const double* a, unsigned long long pol)
-{
-  double v;
-  asm volatile("ld.global.nc.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(v) : "l"(a), "l"(pol));
-  return v;
-}
-
-// pol = 0: plain read-only load
-__device__ __forceinline__ void tp_pull_at(const double* __restrict__ node, const SlabGeom& g, double (&f)[9], unsigned long long pol = 0ull)
+__device__ __forceinline__ void tp_pull_at(const double* __restrict__ node, const SlabGeom& g, double (&f)[9])
 {
 #pragma unroll
-  for (int q = 0; q < 9; q++)
-  {
-    const double* a = node + ((long long)q * g.plane - (long long)CX(q) * g.pitch - CY(q));
-#if LBM_TP_HINTS
-    f[q] = ld_l2_hint(a, pol);
-#else
-    f[q] = __ldg(a);
-#endif
-  }
+  for (int q = 0; q < 9; q++) f[q] = __ldg(node + ((long long)q * g.plane - (long long)CX(q) * g.pitch - CY(q)));
 }
 
 template <int MODE>
@@ -424,14 +387,8 @@ __device__ __forceinline__ void tp_ring_stencil(const double* __restrict__ sm, i
 //               work of B (software pipelining, 36 more live registers).
 // Resident blocks per SM the register allocation aims at.  Measured on B200 at 8192^2 (MRTCG, pipelined):
 // 2 blocks (208 regs) 12.1 GLUPS, 3 blocks (168 regs, no spills) 12.9 GLUPS, 4 blocks (128 regs, spills) 8.0 GLUPS.
-#ifndef LBM_TPF_MINB
-#define LBM_TPF_MINB 3
-#endif
-#ifndef LBM_TPF_MINB_RK
-#define LBM_TPF_MINB_RK 3
-#endif
 template <int MODEL, bool PIPE>
-__global__ void __launch_bounds__(TPF_NT, MODEL == TP_MRTCG ? (PIPE ? LBM_TPF_MINB : LBM_TPF_MINB + 1) : LBM_TPF_MINB_RK)
+__global__ void __launch_bounds__(TPF_NT, MODEL == TP_MRTCG ? (PIPE ? 3 : 4) : 3)
 k_tp_fused(const double* __restrict__ rsrc, const double* __restrict__ bsrc, double* __restrict__ rdst,
            double* __restrict__ bdst, const SlabGeom g, const MomGeom mg, const double* __restrict__ mom, const TpParams p,
            const unsigned char* __restrict__ rowflag, int rows_per_block, int band_lo, int band_jump)
@@ -455,17 +412,11 @@ k_tp_fused(const double* __restrict__ rsrc, const double* __restrict__ bsrc, dou
   const double* pb = bsrc + o0;
   const long long back = (long long)LAG * g.pitch;
 
-#if LBM_TP_HINTS
-  const unsigned long long pol_first = l2_policy_evict_last(), pol_second = l2_policy_evict_first();
-#else
-  const unsigned long long pol_first = 0ull, pol_second = 0ull;
-#endif
-
   auto collide_row = [&](int sc) {
     // the second pull of this row (an L2 hit) first, so that its latency hides under the stencil arithmetic
     double fr[9], fb[9];
-    tp_pull_at(pr - back, g, fr, pol_second);
-    tp_pull_at(pb - back, g, fb, pol_second);
+    tp_pull_at(pr - back, g, fr);
+    tp_pull_at(pb - back, g, fb);
     TpStencil st;
     tp_ring_stencil<MODEL>(sm, sc, t, st);
     const double rr = S(C::F_RR, sc, t), rb = S(C::F_RB, sc, t);
@@ -476,13 +427,8 @@ k_tp_fused(const double* __restrict__ rsrc, const double* __restrict__ bsrc, dou
 #pragma unroll
     for (int q = 0; q < 9; q++)
     {
-#if LBM_TP_HINTS >= 2
-      asm volatile("st.global.L2::cache_hint.f64 [%0], %1, %2;" ::"l"(wr + (long long)q * g.plane), "d"(fr[q]), "l"(pol_second) : "memory");
-      asm volatile("st.global.L2::cache_hint.f64 [%0], %1, %2;" ::"l"(wb + (long long)q * g.plane), "d"(fb[q]), "l"(pol_second) : "memory");
-#else
       wr[(long long)q * g.plane] = fr[q];
       wb[(long long)q * g.plane] = fb[q];
-#endif
     }
   };
 
@@ -518,8 +464,8 @@ k_tp_fused(const double* __restrict__ rsrc, const double* __restrict__ bsrc, dou
       }
       else
       {
-        tp_pull_at(pr, g, fr, pol_first);
-        tp_pull_at(pb, g, fb, pol_first);
+        tp_pull_at(pr, g, fr);
+        tp_pull_at(pb, g, fb);
       }
     }
     // ---- B (pipelined): collision of row r - LAG
@@ -1123,63 +1069,67 @@ __global__ void k_tp_write_u(double* __restrict__ mom, const SlabGeom g, const M
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-static int csf_configure();
-
-int tp_create(lbm_domain* d)
+// f(std::integral_constant<int, MODEL>()) for the domain's model: TP_RK, or TP_MRTCG for the others (TP_CSF's export and
+// import passes are MRTCG's: the export only pulls, and an import carries no interfacial tension)
+template <class F>
+static int with_model(const TwoPhaseState* tp, F&& f)
 {
-  TwoPhaseState* tp = new TwoPhaseState();
-  d->tp = tp;
-  tp->model = d->cfg.model == LBM_MODEL_MRTCG ? TP_MRTCG : (d->cfg.model == LBM_MODEL_MRT_CSF ? TP_CSF : TP_RK);
-  tp->mg.pm = ((d->g.Y + 4 + 15) / 16) * 16;
-  tp->mg.mplane = (long long)(d->g.Xl + 4) * tp->mg.pm;
-  const size_t bytes = sizeof(double) * M_COUNT * tp->mg.mplane;
-  LBM_CUDA(cudaMalloc(&tp->mom, bytes));
-  LBM_CUDA(cudaMemset(tp->mom, 0, bytes));
-  TpParams& p = tp->p;
-  const lbm_config& c = d->cfg;
-  if (!(c.red.rho_0 > 0.0) || !(c.blue.rho_0 > 0.0) || !(c.delta > 0.0))
+  if (tp->model == TP_RK) return f(std::integral_constant<int, TP_RK>());
+  return f(std::integral_constant<int, TP_MRTCG>());
+}
+
+// The row-marching kernels a switch can select.  All instantiations of one family have the same parameters, so one table
+// gives tp_create the attributes to set and the kernel to resolve, and the step its launch.
+struct TpKernel
+{
+  int model;
+  bool staged, stash;  // k_tp_staged (with the tensor-memory stash), or k_tp_fused
+  int ns;              // k_tp_staged: stage slots
+  bool pipe;           // k_tp_fused: the software-pipelined variant
+  decltype(&k_tp_fused<TP_MRTCG, true>) kernel;
+  size_t smem;
+  int warmup_rows;     // band height: pick_band_rows with this many warm-up rows per band
+};
+template <int MODEL, bool PIPE>
+static TpKernel tp_fused_kernel() { return {MODEL, false, false, 0, PIPE, k_tp_fused<MODEL, PIPE>, TpFused<MODEL>::SMEM, 2 * TpFused<MODEL>::H}; }
+template <int MODEL, int NS, int MINB, bool STASH>
+static TpKernel tp_staged_kernel() { return {MODEL, true, STASH, NS, false, k_tp_staged<MODEL, NS, MINB, STASH>, TpStaged<MODEL, NS>::SMEM, 2 * TpFused<MODEL>::H}; }
+static const TpKernel tp_kernels[] = {
+    tp_fused_kernel<TP_MRTCG, false>(), tp_fused_kernel<TP_MRTCG, true>(), tp_fused_kernel<TP_RK, false>(), tp_fused_kernel<TP_RK, true>(),
+    tp_staged_kernel<TP_MRTCG, 4, 2, false>(), tp_staged_kernel<TP_MRTCG, 5, 2, false>(), tp_staged_kernel<TP_MRTCG, 6, 2, false>(),
+    tp_staged_kernel<TP_RK, 3, 3, false>(), tp_staged_kernel<TP_RK, 4, 2, false>(), tp_staged_kernel<TP_RK, 5, 2, false>(), tp_staged_kernel<TP_RK, 6, 2, false>(),
+    tp_staged_kernel<TP_MRTCG, 2, 4, true>(), tp_staged_kernel<TP_MRTCG, 3, 3, true>(), tp_staged_kernel<TP_MRTCG, 4, 2, true>(),
+    tp_staged_kernel<TP_RK, 2, 4, true>(), tp_staged_kernel<TP_RK, 3, 3, true>(), tp_staged_kernel<TP_RK, 4, 2, true>()};
+
+// the switches' kernel (LBM_TP_PIPE counts only when LBM_TP_STAGED=0)
+static const TpKernel* tp_pick_kernel(int model, bool staged, bool stash, int stages, bool pipe)
+{
+  int ns = 0;
+  if (staged)
   {
-    set_error("two-phase model: red/blue initial_density and delta must be positive");
-    return LBM_ERR_INVALID;
+    // stage slots.  With the stash: the rows in flight only (2 .. 4).  Without it: H + 1 resident rows + the rows in flight
+    // (H + 2 .. 6).  stages <= 0: the model's default
+    const int H = model == TP_MRTCG ? TpFused<TP_MRTCG>::H : TpFused<TP_RK>::H;
+    ns = stash ? std::clamp(stages > 0 ? stages : (model == TP_MRTCG ? 3 : 4), 2, 4) : std::clamp(stages > 0 ? stages : 5, H + 2, 6);
+    pipe = false;
   }
-  tp_fill_params(c, (TpModel)tp->model, p);
-  if (tp->model == TP_CSF)
-  {
-    const size_t ab = sizeof(double) * 4 * tp->mg.mplane;
-    LBM_CUDA(cudaMalloc(&tp->aux, ab));
-    LBM_CUDA(cudaMemset(tp->aux, 0, ab));
-    if (const char* e = getenv("LBM_CSF_FUSED")) tp->csf_fused = atoi(e) != 0;
-    if (const char* e = getenv("LBM_CSF_PIPE")) tp->csf_pipe = atoi(e) != 0;
-    if (const char* e = getenv("LBM_CSF_STAGED")) tp->csf_staged = atoi(e);
-    if (tp->csf_fused)
-    {
-      LBM_CUDA(cudaMalloc(&tp->aux_next, ab));
-      LBM_CUDA(cudaMemset(tp->aux_next, 0, ab));
-    }
-  }
-  LBM_CUDA(cudaFuncSetAttribute(k_tp_fused<TP_MRTCG, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TpFused<TP_MRTCG>::SMEM));
-  LBM_CUDA(cudaFuncSetAttribute(k_tp_fused<TP_MRTCG, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TpFused<TP_MRTCG>::SMEM));
-  LBM_CUDA(cudaFuncSetAttribute(k_tp_fused<TP_RK, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TpFused<TP_RK>::SMEM));
-  LBM_CUDA(cudaFuncSetAttribute(k_tp_fused<TP_RK, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TpFused<TP_RK>::SMEM));
-#define LBM_STAGED_ATTR(MODEL, NS, MINB, STASH)                                                                                             \
-  LBM_CUDA(cudaFuncSetAttribute(k_tp_staged<MODEL, NS, MINB, STASH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TpStaged<MODEL, NS>::SMEM)); \
-  LBM_CUDA(cudaFuncSetAttribute(k_tp_staged<MODEL, NS, MINB, STASH>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))
-  LBM_STAGED_ATTR(TP_MRTCG, 4, 2, false); LBM_STAGED_ATTR(TP_MRTCG, 5, 2, false); LBM_STAGED_ATTR(TP_MRTCG, 6, 2, false);
-  LBM_STAGED_ATTR(TP_RK, 3, 3, false); LBM_STAGED_ATTR(TP_RK, 4, 2, false); LBM_STAGED_ATTR(TP_RK, 5, 2, false); LBM_STAGED_ATTR(TP_RK, 6, 2, false);
-  LBM_STAGED_ATTR(TP_MRTCG, 2, 4, true); LBM_STAGED_ATTR(TP_MRTCG, 3, 3, true); LBM_STAGED_ATTR(TP_MRTCG, 4, 2, true);
-  LBM_STAGED_ATTR(TP_RK, 2, 4, true); LBM_STAGED_ATTR(TP_RK, 3, 3, true); LBM_STAGED_ATTR(TP_RK, 4, 2, true);
-#undef LBM_STAGED_ATTR
-  LBM_TRY(csf_configure());
-  if (const char* e = getenv("LBM_TP_PIPE")) tp->pipe = atoi(e) != 0;
-  if (const char* e = getenv("LBM_TP_STAGED")) tp->staged = atoi(e) != 0;
-  if (const char* e = getenv("LBM_TP_NS")) tp->stages = atoi(e);
-  // MRTCG (H = 2): the stash frees shared memory for a third block per SM (+17 %).  RK (H = 1) runs two blocks either way
-  // and is 1 % faster with its two resident rows left in the stage slots
-  tp->stash = tp->model == TP_MRTCG;
-  if (const char* e = getenv("LBM_TP_STASH")) tp->stash = atoi(e) != 0;
-  if (const char* e = getenv("LBM_TP_RPB")) tp->rpb_override = atoi(e);
-  if (const char* e = getenv("LBM_TP_OVERLAP")) tp->ring_overlap = atoi(e) != 0;  // (off by default: see tp_steps_ring)
-  return LBM_OK;
+  else stash = false;
+  for (const TpKernel& k : tp_kernels)
+    if (k.model == model && k.staged == staged && k.stash == stash && k.ns == ns && k.pipe == pipe) return &k;
+  return nullptr;
+}
+
+// band height of a row-marching kernel, once per rule set: LBM_TP_RPB, else from the occupancy of the kernel that runs
+// (warmup_rows = 0: 64 rows)
+template <class K>
+static int band_rows(lbm_domain* d, int strips, const K& k)
+{
+  TwoPhaseState* tp = d->tp;
+  if (tp->rows_per_block <= 0)
+    tp->rows_per_block = tp->rpb_override > 0 ? std::min(128, tp->rpb_override)  // the kernels stage <= 128 + 2H row flags
+                         : k.warmup_rows > 0 ? pick_band_rows(d->g.Xl, strips, resident_blocks_of(d, k.kernel, k.smem), k.warmup_rows)
+                                             : 64;
+  return tp->rows_per_block;
 }
 
 double* tp_moment_planes(lbm_domain* d, int* pm, long long* mplane)
@@ -1352,45 +1302,21 @@ static int tp_launch_fused(lbm_domain* d, int part = TP_BANDS_ALL)
   const int Yi = d->g.Y - 2;
   if (Yi > 0)
   {
-    const int strips = cdiv(Yi, C::USEFUL);
-    // one launcher per kernel variant: band height from that variant's occupancy (once per rule set), then the launch
-    auto run = [&](auto kernel, size_t smem) {
-      if (tp->rows_per_block <= 0)
-        tp->rows_per_block = tp->rpb_override > 0 ? std::min(128, tp->rpb_override)  // the kernels stage <= 128 + 2H row flags
-                                                  : pick_band_rows(d->g.Xl, strips, resident_blocks_of(d, kernel, smem), 2 * C::H);
-      if (part == TP_BANDS_NONE) return;
+    const int strips = cdiv(Yi, C::USEFUL), rpb = band_rows(d, strips, *tp->kernel);
+    if (part != TP_BANDS_NONE)
+    {
       ProfScope ps(d, LBM_PROF_INTERIOR);
       // grid row j works on band j < band_lo ? j : j + band_jump
-      const int nb = cdiv(d->g.Xl, tp->rows_per_block), k_hi = tp_edge_bands_hi(d);
+      const int nb = cdiv(d->g.Xl, rpb), k_hi = tp_edge_bands_hi(d);
       int ny = nb, band_lo = 0, band_jump = 0;
       if (part == TP_BANDS_EDGE) { ny = 1 + k_hi; band_lo = 1; band_jump = nb - k_hi - 1; }
       if (part == TP_BANDS_INTERIOR) { ny = nb - 1 - k_hi; band_jump = 1; }
       dim3 grid(strips, ny);
-      kernel<<<grid, TPF_NT, smem, d->stream>>>(d->buf[0][s], d->buf[1][s], d->buf[0][t], d->buf[1][t], d->g, tp->mg, tp->mom, tp->p,
-                                                tp->d_rowflag, tp->rows_per_block, band_lo, band_jump);
+      auto k = tp->kernel->kernel;
+      k<<<grid, TPF_NT, tp->kernel->smem, d->stream>>>(d->buf[0][s], d->buf[1][s], d->buf[0][t], d->buf[1][t], d->g, tp->mg, tp->mom, tp->p,
+                                                      tp->d_rowflag, rpb, band_lo, band_jump);
       d->launches++;
-    };
-    if (tp->staged)
-    {
-      // stage slots.  Without the stash: H + 1 resident rows + the rows in flight (default 5).  With it: rows in flight only
-      const int ns = tp->stash ? std::max(2, tp->stages > 0 ? tp->stages : (MODEL == TP_MRTCG ? 3 : 4))
-                               : std::max(C::H + 2, tp->stages > 0 ? tp->stages : 5);
-      if (tp->stash)
-      {
-        if (ns <= 2) run(k_tp_staged<MODEL, 2, 4, true>, TpStaged<MODEL, 2>::SMEM);
-        else if (ns == 3) run(k_tp_staged<MODEL, 3, 3, true>, TpStaged<MODEL, 3>::SMEM);
-        else run(k_tp_staged<MODEL, 4, 2, true>, TpStaged<MODEL, 4>::SMEM);
-      }
-      else if (ns <= 3)
-      {
-        if constexpr (C::H + 2 <= 3) run(k_tp_staged<MODEL, 3, 3, false>, TpStaged<MODEL, 3>::SMEM);
-      }
-      else if (ns == 4) run(k_tp_staged<MODEL, 4, 2, false>, TpStaged<MODEL, 4>::SMEM);
-      else if (ns == 5) run(k_tp_staged<MODEL, 5, 2, false>, TpStaged<MODEL, 5>::SMEM);
-      else run(k_tp_staged<MODEL, 6, 2, false>, TpStaged<MODEL, 6>::SMEM);
     }
-    else if (tp->pipe) run(k_tp_fused<MODEL, true>, C::SMEM);
-    else run(k_tp_fused<MODEL, false>, C::SMEM);
   }
   // listed nodes after the bands that hold them (a band writes every node of its rows' interior columns; with the bands split,
   // tp_ring_overlap_ok has checked that only the edge bands hold any)
@@ -1419,10 +1345,10 @@ static int tp_phase_pre(lbm_domain* d)
   if (tp->n_region > 0 || d->nb > 0)
   {
     const int blocks = cdiv(tp->n_region, 128) + cdiv(d->nb, 128);
-    if (tp->model == TP_MRTCG)
-      k_tp_moments_region<TP_MRTCG><<<blocks, 128, 0, d->stream>>>(d->buf[0][s], d->buf[1][s], d->g, tp->mg, tp->mom, tp->p, tp->d_region, tp->n_region, table_of(d));
-    else
-      k_tp_moments_region<TP_RK><<<blocks, 128, 0, d->stream>>>(d->buf[0][s], d->buf[1][s], d->g, tp->mg, tp->mom, tp->p, tp->d_region, tp->n_region, table_of(d));
+    with_model(tp, [&](auto M) {
+      k_tp_moments_region<M><<<blocks, 128, 0, d->stream>>>(d->buf[0][s], d->buf[1][s], d->g, tp->mg, tp->mom, tp->p, tp->d_region, tp->n_region, table_of(d));
+      return LBM_OK;
+    });
     d->launches++;
   }
   LBM_TRY(tp_pad(d));
@@ -1434,16 +1360,7 @@ static int tp_phase_pre(lbm_domain* d)
 static int tp_phase_main(lbm_domain* d)
 {
   TwoPhaseState* tp = d->tp;
-  if (d->post_stream)
-  {
-    if (tp->model == TP_MRTCG) LBM_TRY((tp_launch_collide<TP_MRTCG, MODE_LOCAL>(d)));
-    else LBM_TRY((tp_launch_collide<TP_RK, MODE_LOCAL>(d)));
-  }
-  else
-  {
-    if (tp->model == TP_MRTCG) LBM_TRY(tp_launch_fused<TP_MRTCG>(d));
-    else LBM_TRY(tp_launch_fused<TP_RK>(d));
-  }
+  LBM_TRY(with_model(tp, [&](auto M) { return d->post_stream ? tp_launch_collide<M, MODE_LOCAL>(d) : tp_launch_fused<M>(d); }));
   d->cur ^= 1;
   d->post_stream = false;
   tp->planes_full = false;
@@ -1520,11 +1437,7 @@ bool tp_ring_overlap_ok(lbm_domain* d)
   TwoPhaseState* tp = d->tp;
   if (!tp || tp->model == TP_CSF || !tp->ring_overlap || !comm_active(d) || d->post_stream || d->g.Xl < 16 || d->g.Y < 3) return false;
   if (tp_build_region(d) != LBM_OK) return false;
-  if (tp->rows_per_block <= 0)
-  {
-    if (tp->model == TP_MRTCG) tp_launch_fused<TP_MRTCG>(d, TP_BANDS_NONE);
-    else tp_launch_fused<TP_RK>(d, TP_BANDS_NONE);
-  }
+  if (tp->rows_per_block <= 0) with_model(tp, [&](auto M) { return tp_launch_fused<M>(d, TP_BANDS_NONE); });
   const int rpb = tp->rows_per_block, nb = cdiv(d->g.Xl, rpb);
   if (rpb < 4 || nb < 4) return false;
   // a band overwrites the listed nodes of its rows' interior columns until the listed-node kernel has run: interior bands must hold none
@@ -1576,30 +1489,10 @@ static int tp_steps_ring_t(lbm_domain* d, int n)
 
 int tp_steps_ring(lbm_domain* d, int n)
 {
-  return d->tp->model == TP_MRTCG ? tp_steps_ring_t<TP_MRTCG>(d, n) : tp_steps_ring_t<TP_RK>(d, n);
+  return with_model(d->tp, [&](auto M) { return tp_steps_ring_t<M>(d, n); });
 }
 
-static int csf_step(lbm_domain* d);
 static int csf_fill_planes(lbm_domain* d);
-
-int tp_step(lbm_domain* d)
-{
-  if (d->tp->model == TP_CSF) return csf_step(d);
-  LBM_TRY(tp_phase_pre(d));
-  if (!d->post_stream)
-  {
-    ProfScope ps(d, LBM_PROF_MOMENTS);
-    LBM_TRY(comm_exchange_moments(d));  // two plane rows across every cut (NCCL); nothing on a single slab
-  }
-  LBM_TRY(tp_phase_main(d));
-  {
-    // the next step pulls from the buffer just written: its ghost rows
-    ProfScope ps(d, LBM_PROF_GHOST);
-    if (comm_active(d)) LBM_TRY(comm_exchange(d, d->cur, d->stream));
-    else LBM_TRY(wrap_ghost_rows_local(d, d->cur, d->stream));
-  }
-  return LBM_OK;
-}
 
 // two rows of `nplanes` planes (moment-plane geometry) from the linked neighbours across every INTERNAL cut (the global
 // edge replicates): the five moment planes, or the CSF model's normal field
@@ -1632,69 +1525,6 @@ static int tp_link_halo_planes(lbm_domain* d, double* TwoPhaseState::*field, int
   return LBM_OK;
 }
 
-static int tp_link_halo(lbm_domain* d) { return tp_link_halo_planes(d, &TwoPhaseState::mom, M_COUNT); }
-
-static int csf_step_group(lbm_domain* const* ds, int n, int n_steps);
-
-// Linked two-phase slabs in lock step (lbm_step_group): the phases of tp_step interleaved across the slabs, every
-// cross-slab read ordered by events on the slabs' streams:
-//   pre_i   waits until the neighbours finished reading slab i's plane rows (their halo of the step before)
-//   halo_i  waits for the neighbours' pre;   main_i;   ghost_i waits for the neighbours' main
-int tp_step_group(lbm_domain* const* ds, int n, int n_steps)
-{
-  if (ds[0]->tp->model == TP_CSF) return csf_step_group(ds, n, n_steps);
-  auto on = [](lbm_domain* d) { return cudaSetDevice(d->cfg.device); };
-  auto wait_neighbours = [&](lbm_domain* d, cudaEvent_t lbm_domain::*ev) -> int {
-    for (lbm_domain* o : {d->link_lo, d->link_hi})
-      if (o && o != d) LBM_CUDA(cudaStreamWaitEvent(d->stream, o->*ev, 0));
-    return LBM_OK;
-  };
-  for (int i = 0; i < n; i++)
-  {
-    LBM_CUDA(on(ds[i]));
-    LBM_CUDA(cudaEventRecord(ds[i]->ev_begin, ds[i]->stream));
-    LBM_CUDA(cudaEventRecord(ds[i]->ev_packet, ds[i]->stream));  // "nobody is reading my planes"
-  }
-  for (int s = 0; s < n_steps; s++)
-  {
-    for (int i = 0; i < n; i++)
-    {
-      LBM_CUDA(on(ds[i]));
-      LBM_TRY(wait_neighbours(ds[i], &lbm_domain::ev_packet));
-      LBM_TRY(tp_phase_pre(ds[i]));
-      LBM_CUDA(cudaEventRecord(ds[i]->ev_ready, ds[i]->stream));
-    }
-    for (int i = 0; i < n; i++)
-    {
-      LBM_CUDA(on(ds[i]));
-      LBM_TRY(wait_neighbours(ds[i], &lbm_domain::ev_ready));
-      LBM_TRY(tp_link_halo(ds[i]));
-      LBM_CUDA(cudaEventRecord(ds[i]->ev_packet, ds[i]->stream));
-    }
-    for (int i = 0; i < n; i++)
-    {
-      LBM_CUDA(on(ds[i]));
-      LBM_TRY(tp_phase_main(ds[i]));
-      LBM_CUDA(cudaEventRecord(ds[i]->ev_stage, ds[i]->stream));
-    }
-    for (int i = 0; i < n; i++)
-    {
-      lbm_domain* d = ds[i];
-      LBM_CUDA(on(d));
-      LBM_TRY(wait_neighbours(d, &lbm_domain::ev_stage));
-      ProfScope ps(d, LBM_PROF_GHOST);
-      if (d->link_lo || d->link_hi) LBM_TRY(link_exchange(d, d->cur, d->stream));
-      else LBM_TRY(wrap_ghost_rows_local(d, d->cur, d->stream));
-    }
-  }
-  for (int i = 0; i < n; i++)
-  {
-    LBM_CUDA(on(ds[i]));
-    LBM_CUDA(cudaEventRecord(ds[i]->ev_end, ds[i]->stream));
-  }
-  return LBM_OK;
-}
-
 // moments of every own node of the current state into the planes (diagnostics: lbm_get_moments /
 // lbm_get_phase after fused steps).  No exchange: the halo cells are rebuilt by the next step.
 static int tp_fill_planes(lbm_domain* d)
@@ -1702,8 +1532,7 @@ static int tp_fill_planes(lbm_domain* d)
   TwoPhaseState* tp = d->tp;
   if (tp->planes_full || d->post_stream) return LBM_OK;
   if (tp->model == TP_CSF) return csf_fill_planes(d);
-  if (tp->model == TP_MRTCG) LBM_TRY(tp_launch_moments<TP_MRTCG>(d, d->cur, nullptr, nullptr));
-  else LBM_TRY(tp_launch_moments<TP_RK>(d, d->cur, nullptr, nullptr));
+  LBM_TRY(with_model(tp, [&](auto M) { return tp_launch_moments<M>(d, d->cur, nullptr, nullptr); }));
   tp->planes_full = true;
   return LBM_OK;
 }
@@ -1736,8 +1565,7 @@ int tp_export(lbm_domain* d)
     return LBM_OK;
   }
   // (with output pointers the pass only pulls: no model arithmetic)
-  if (d->tp->model != TP_RK) return tp_launch_moments<TP_MRTCG>(d, d->cur, d->d_aos[0], d->d_aos[1]);
-  return tp_launch_moments<TP_RK>(d, d->cur, d->d_aos[0], d->d_aos[1]);
+  return with_model(d->tp, [&](auto M) { return tp_launch_moments<M>(d, d->cur, d->d_aos[0], d->d_aos[1]); });
 }
 
 int tp_stage_moments(lbm_domain* d, double* stage)
@@ -1755,10 +1583,10 @@ int tp_stage_moments(lbm_domain* d, double* stage)
 int tp_refresh_moments(lbm_domain* d)
 {
   const long long N = (long long)d->g.Xl * d->g.Y;
-  if (d->tp->model != TP_RK)  // TP_CSF: an import carries no interfacial tension (u = j / rho + Fg / (2 rho))
-    k_tp_moments_local<TP_MRTCG><<<cdiv(N, 256), 256, 0, d->stream>>>(d->buf[0][d->cur], d->buf[1][d->cur], d->g, d->tp->mg, d->tp->mom, d->tp->p);
-  else
-    k_tp_moments_local<TP_RK><<<cdiv(N, 256), 256, 0, d->stream>>>(d->buf[0][d->cur], d->buf[1][d->cur], d->g, d->tp->mg, d->tp->mom, d->tp->p);
+  with_model(d->tp, [&](auto M) {  // TP_CSF: an import carries no interfacial tension (u = j / rho + Fg / (2 rho))
+    k_tp_moments_local<M><<<cdiv(N, 256), 256, 0, d->stream>>>(d->buf[0][d->cur], d->buf[1][d->cur], d->g, d->tp->mg, d->tp->mom, d->tp->p);
+    return LBM_OK;
+  });
   d->launches++;
   d->tp->planes_full = true;
   LBM_TRY(tp_pad(d));
@@ -2083,12 +1911,6 @@ k_csf_fused(const double* __restrict__ rsrc, const double* __restrict__ bsrc, do
   const bool col_plane = y < 1 || y > g.Y - 2;      // listed edge columns and the padding
   const bool normal_thread = t >= 2 && t < NT - 2;  // has the phase of its columns y-2 .. y+2 in the ring
   const bool collider = t >= HC && t < NT - HC && y >= 1 && y <= g.Y - 2;
-
-#if LBM_TP_HINTS
-  const unsigned long long pol_first = l2_policy_evict_last(), pol_second = l2_policy_evict_first();
-#else
-  const unsigned long long pol_first = 0ull, pol_second = 0ull;
-#endif
   __shared__ unsigned char sflag[128 + 16];  // flags of rows xb-4 .. xe+4 (outside the slab: everything from the planes)
   for (int k = t; k < xe - xb + 9; k += NT)
   {
@@ -2153,8 +1975,8 @@ k_csf_fused(const double* __restrict__ rsrc, const double* __restrict__ bsrc, do
       if (x >= xb && x < xe && collider)
       {
         double fr[9], fb[9];
-        tp_pull_at(rsrc + node_off(g, x, y), g, fr, pol_second);
-        tp_pull_at(bsrc + node_off(g, x, y), g, fb, pol_second);
+        tp_pull_at(rsrc + node_off(g, x, y), g, fr);
+        tp_pull_at(bsrc + node_off(g, x, y), g, fb);
         const long long k = mom_off(mg, x, y);
         double rr, rb, ux, uy, ph;
         // the same arithmetic on the same inputs as stage A / the pre-pass: identical values, no ring rows for them
@@ -2209,13 +2031,8 @@ k_csf_fused(const double* __restrict__ rsrc, const double* __restrict__ bsrc, do
 #pragma unroll
         for (int q = 0; q < 9; q++)
         {
-#if LBM_TP_HINTS >= 2
-          asm volatile("st.global.L2::cache_hint.f64 [%0], %1, %2;" ::"l"(rdst + q * g.plane + o), "d"(fr[q]), "l"(pol_second) : "memory");
-          asm volatile("st.global.L2::cache_hint.f64 [%0], %1, %2;" ::"l"(bdst + q * g.plane + o), "d"(fb[q]), "l"(pol_second) : "memory");
-#else
           rdst[q * g.plane + o] = fr[q];
           bdst[q * g.plane + o] = fb[q];
-#endif
         }
       }
     }
@@ -2240,8 +2057,8 @@ k_csf_fused(const double* __restrict__ rsrc, const double* __restrict__ bsrc, do
       }
       else
       {
-        tp_pull_at(rsrc + node_off(g, r, y), g, fr, pol_first);
-        tp_pull_at(bsrc + node_off(g, r, y), g, fb, pol_first);
+        tp_pull_at(rsrc + node_off(g, r, y), g, fr);
+        tp_pull_at(bsrc + node_off(g, r, y), g, fb);
         fsx = aux[A_FX * mg.mplane + k];
         fsy = aux[A_FY * mg.mplane + k];
       }
@@ -2587,17 +2404,28 @@ k_csf_staged(const double* __restrict__ rsrc, const double* __restrict__ bsrc, d
   if constexpr (STASH) tmem_free<C::TMEM_COLS>(tmem);
 }
 
-static int csf_configure()
+// the single pass's row-marching kernels, as tp_kernels for MRTCG / RK
+struct CsfKernel
 {
-  LBM_CUDA(cudaFuncSetAttribute(k_csf_collide_ring<MODE_LOCAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CsfRing::SMEM));
-  LBM_CUDA(cudaFuncSetAttribute(k_csf_collide_ring<MODE_PULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CsfRing::SMEM));
-  LBM_CUDA(cudaFuncSetAttribute(k_csf_fused<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CsfFused::SMEM));
-  LBM_CUDA(cudaFuncSetAttribute(k_csf_fused<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CsfFused::SMEM));
-  LBM_CUDA(cudaFuncSetAttribute(k_csf_staged<3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CsfStaged<3>::SMEM));
-  LBM_CUDA(cudaFuncSetAttribute(k_csf_staged<7, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CsfStaged<7>::SMEM));
-  LBM_CUDA(cudaFuncSetAttribute(k_csf_staged<3, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  LBM_CUDA(cudaFuncSetAttribute(k_csf_staged<7, false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  return LBM_OK;
+  int staged;  // LBM_CSF_STAGED: 2 = k_csf_staged with the tensor-memory stash, 1 = without it, 0 (or any other value) = k_csf_fused
+  bool pipe;   // k_csf_fused: the software-pipelined variant (LBM_CSF_PIPE)
+  decltype(&k_csf_fused<false>) kernel;
+  size_t smem;
+  int warmup_rows;  // band height: pick_band_rows with this many warm-up rows per band, 0 = 64 rows
+};
+static const CsfKernel csf_kernels[] = {{0, false, k_csf_fused<false>, CsfFused::SMEM, 0},
+                                        {0, true, k_csf_fused<true>, CsfFused::SMEM, 0},
+                                        {1, false, k_csf_staged<7, false>, CsfStaged<7>::SMEM, 8},
+                                        {2, false, k_csf_staged<3, true>, CsfStaged<3>::SMEM, 8}};
+
+// the switches' kernel (LBM_CSF_PIPE counts only for k_csf_fused)
+static const CsfKernel* csf_pick_kernel(int staged, bool pipe)
+{
+  if (staged != 1 && staged != 2) staged = 0;
+  else pipe = false;
+  for (const CsfKernel& k : csf_kernels)
+    if (k.staged == staged && k.pipe == pipe) return &k;
+  return nullptr;
 }
 
 // rho_r, rho_b, u (with the stored interfacial tension), phase of the current post-stream state into the planes
@@ -2737,14 +2565,14 @@ static int csf_build_lists(lbm_domain* d)
   LBM_CUDA(cudaMemcpy(tp->d_csf_list4, list4.data(), sizeof(int) * list4.size(), cudaMemcpyHostToDevice));
   LBM_CUDA(cudaMemcpy(tp->d_csf_list2, list2.data(), sizeof(int) * list2.size(), cudaMemcpyHostToDevice));
   tp->csf_lists_dirty = false;
-  tp->csf_rows = 0;
+  tp->rows_per_block = 0;
   return LBM_OK;
 }
 
 static bool csf_can_fuse(const lbm_domain* d)
 {
   // monolithic domains and the slabs of an NCCL ring (two 2-row halos between the pre-pass stages, like the three-pass
-  // step) or of a linked group (csf_step_group interleaves the same three stages)
+  // step) or of a linked group (tp_step_group interleaves the same three stages)
   const bool whole = d->cfg.x0 == 0 && d->cfg.x1 == d->cfg.X, linked = d->link_lo || d->link_hi;
   return d->tp->csf_fused && !d->post_stream && (whole || comm_active(d) || linked) && d->g.Xl >= 8 && d->g.Y >= 12;
 }
@@ -2791,28 +2619,11 @@ static int csf_fused_collide(lbm_domain* d)
   if (Yi > 0)
   {
     ProfScope ps(d, LBM_PROF_INTERIOR);
-    const int strips = cdiv(Yi, CsfFused::USEFUL);
-    auto band_rows = [&](auto kernel, size_t smem) {
-      if (tp->rpb_override > 0) return std::min(128, tp->rpb_override);
-      if (tp->csf_rows <= 0) tp->csf_rows = pick_band_rows(d->g.Xl, strips, resident_blocks_of(d, kernel, smem), 8);
-      return tp->csf_rows;
-    };
-    int rpb = tp->rpb_override > 0 ? std::min(128, tp->rpb_override) : 64;
-    if (tp->csf_staged == 2) rpb = band_rows(k_csf_staged<3, true>, CsfStaged<3>::SMEM);
-    else if (tp->csf_staged == 1) rpb = band_rows(k_csf_staged<7, false>, CsfStaged<7>::SMEM);
+    const int strips = cdiv(Yi, CsfFused::USEFUL), rpb = band_rows(d, strips, *tp->csf_kernel);
     dim3 grid(strips, cdiv(d->g.Xl, rpb));
-    if (tp->csf_staged == 2)
-      k_csf_staged<3, true><<<grid, TPF_NT, CsfStaged<3>::SMEM, d->stream>>>(d->buf[0][s], d->buf[1][s], d->buf[0][t], d->buf[1][t], d->g, tp->mg,
-                                                                            tp->mom, tp->aux, tp->aux_next, tp->p, tp->d_csf_flags, rpb);
-    else if (tp->csf_staged == 1)
-      k_csf_staged<7, false><<<grid, TPF_NT, CsfStaged<7>::SMEM, d->stream>>>(d->buf[0][s], d->buf[1][s], d->buf[0][t], d->buf[1][t], d->g, tp->mg,
-                                                                             tp->mom, tp->aux, tp->aux_next, tp->p, tp->d_csf_flags, rpb);
-    else if (tp->csf_pipe)
-      k_csf_fused<true><<<grid, TPF_NT, CsfFused::SMEM, d->stream>>>(d->buf[0][s], d->buf[1][s], d->buf[0][t], d->buf[1][t], d->g, tp->mg,
-                                                                    tp->mom, tp->aux, tp->aux_next, tp->p, tp->d_csf_flags, rpb);
-    else
-      k_csf_fused<false><<<grid, TPF_NT, CsfFused::SMEM, d->stream>>>(d->buf[0][s], d->buf[1][s], d->buf[0][t], d->buf[1][t], d->g, tp->mg,
-                                                                     tp->mom, tp->aux, tp->aux_next, tp->p, tp->d_csf_flags, rpb);
+    auto k = tp->csf_kernel->kernel;
+    k<<<grid, TPF_NT, tp->csf_kernel->smem, d->stream>>>(d->buf[0][s], d->buf[1][s], d->buf[0][t], d->buf[1][t], d->g, tp->mg, tp->mom, tp->aux,
+                                                         tp->aux_next, tp->p, tp->d_csf_flags, rpb);
     d->launches++;
   }
   if (d->nb > 0)
@@ -2833,84 +2644,107 @@ static int csf_fused_collide(lbm_domain* d)
 // neighbour still copies this step's NORMAL rows out of `aux` after this slab's collision has been enqueued.
 static void csf_fused_swap(lbm_domain* d) { std::swap(d->tp->aux, d->tp->aux_next); }
 
-static int csf_step_fused(lbm_domain* d)
+// ---- one two-phase step as three stages.  A stage takes two halo rows of `nplanes` planes of `halo` across every cut,
+// then runs `phase`.  tp_step runs the stages back to back on one slab (NCCL halos); tp_step_group runs each stage on every
+// linked slab before the next, ordering every cross-slab read by events on the slabs' streams: a stage waits for the
+// neighbours' `wait` event, then records `done`.
+//   MRTCG / RK:  pre (waits until the neighbours have finished reading this slab's plane rows in the step before) ->
+//                moment halo (waits for the neighbours' pre) -> main
+//   CSF:         moments -> moment halo (waits for the neighbours' moments), normals -> normal halo (waits for the
+//                neighbours' normals), collide.  A slab's next moments pass comes after its wait for the neighbours'
+//                collision (ev_stage, before the ghost rows), by which time they have finished copying rows out of its planes.
+struct TpStage
 {
-  LBM_TRY(csf_fused_moments(d));
-  LBM_TRY(comm_exchange_planes(d, d->tp->mom, M_COUNT));  // ring: rows 0, 1 / Xl-2, Xl-1 (whole rows, in the lists) to the neighbours
-  LBM_TRY(csf_fused_normals(d));
-  LBM_TRY(comm_exchange_planes(d, d->tp->aux, 2));
-  LBM_TRY(csf_fused_collide(d));
-  csf_fused_swap(d);
-  ProfScope ps(d, LBM_PROF_GHOST);
-  if (comm_active(d)) return comm_exchange(d, d->cur, d->stream);
-  return wrap_ghost_rows_local(d, d->cur, d->stream);
+  cudaEvent_t lbm_domain::*wait;  // (nullptr: none)
+  double* TwoPhaseState::*halo;   // (nullptr: none)
+  int nplanes;
+  int (*phase)(lbm_domain*);      // (nullptr: none)
+  cudaEvent_t lbm_domain::*done;
+};
+struct TpSchedule
+{
+  TpStage stage[3];
+  bool swap_aux;               // single-pass CSF: the aux sets swap after the collision of every slab (csf_fused_swap)
+  bool import_exchanged;       // MRTCG / RK: an import exchanges the planes it fills, so tp_step skips the halo of the
+                               // step after it (and times the others as moments work)
+};
+static const TpSchedule tp_schedule_mrtcg_rk = {{{&lbm_domain::ev_packet, nullptr, 0, tp_phase_pre, &lbm_domain::ev_ready},
+                                                 {&lbm_domain::ev_ready, &TwoPhaseState::mom, M_COUNT, nullptr, &lbm_domain::ev_packet},
+                                                 {nullptr, nullptr, 0, tp_phase_main, &lbm_domain::ev_stage}},
+                                                false, true};
+static const TpSchedule tp_schedule_csf_fused = {{{nullptr, nullptr, 0, csf_fused_moments, &lbm_domain::ev_ready},
+                                                  {&lbm_domain::ev_ready, &TwoPhaseState::mom, M_COUNT, csf_fused_normals, &lbm_domain::ev_packet},
+                                                  {&lbm_domain::ev_packet, &TwoPhaseState::aux, 2, csf_fused_collide, &lbm_domain::ev_stage}},
+                                                 true, false};
+static const TpSchedule tp_schedule_csf_three = {{{nullptr, nullptr, 0, csf_phase_moments, &lbm_domain::ev_ready},
+                                                  {&lbm_domain::ev_ready, &TwoPhaseState::mom, M_COUNT, csf_phase_normals, &lbm_domain::ev_packet},
+                                                  {&lbm_domain::ev_packet, &TwoPhaseState::aux, 2, csf_phase_collide, &lbm_domain::ev_stage}},
+                                                 false, false};
+
+// the stages of the next step of slabs ds[0 .. n): the same for all of them (CSF: single pass on all slabs or none, since
+// the halo rows a slab sends must be the ones its neighbour's stage expects)
+static const TpSchedule& tp_schedule(lbm_domain* const* ds, int n)
+{
+  if (ds[0]->tp->model != TP_CSF) return tp_schedule_mrtcg_rk;
+  bool fuse = true;
+  for (int i = 0; i < n; i++) fuse = fuse && csf_can_fuse(ds[i]);
+  return fuse ? tp_schedule_csf_fused : tp_schedule_csf_three;
 }
 
-static int csf_step(lbm_domain* d)
+int tp_step(lbm_domain* d)
 {
-  if (csf_can_fuse(d)) return csf_step_fused(d);
+  const TpSchedule& sc = tp_schedule(&d, 1);
   // a three-pass step out of an import does not swap the aux sets while it flips the population buffers: captured step
   // pairs (lbm_use_graph) hold the old pairing of the two.  (Never reached inside a capture: those start in steady state.)
-  if (d->tp->csf_fused && d->post_stream) drop_graphs(d);
-  LBM_TRY(csf_phase_moments(d));
-  LBM_TRY(comm_exchange_planes(d, d->tp->mom, M_COUNT));  // NCCL ring; nothing on a single slab
-  LBM_TRY(csf_phase_normals(d));
-  LBM_TRY(comm_exchange_planes(d, d->tp->aux, 2));
-  LBM_TRY(csf_phase_collide(d));
+  if (&sc == &tp_schedule_csf_three && d->tp->csf_fused && d->post_stream) drop_graphs(d);
+  for (const TpStage& st : sc.stage)
+  {
+    // the halos: NCCL ring (rows 0, 1 / Xl-2, Xl-1 to the neighbours); nothing on a single slab
+    if (st.halo && !sc.import_exchanged) LBM_TRY(comm_exchange_planes(d, d->tp->*st.halo, st.nplanes));
+    else if (st.halo && !d->post_stream)
+    {
+      ProfScope ps(d, LBM_PROF_MOMENTS);
+      LBM_TRY(comm_exchange_planes(d, d->tp->*st.halo, st.nplanes));
+    }
+    if (st.phase) LBM_TRY(st.phase(d));
+  }
+  if (sc.swap_aux) csf_fused_swap(d);
+  // the next step pulls from the buffer just written: its ghost rows
   ProfScope ps(d, LBM_PROF_GHOST);
   if (comm_active(d)) return comm_exchange(d, d->cur, d->stream);
   return wrap_ghost_rows_local(d, d->cur, d->stream);
 }
 
-// linked slabs: the three phases interleaved across the slabs; ev_ready = planes written, ev_packet = normals written,
-// ev_stage = collision done.  A slab's next moments pass comes after its wait for the neighbours' ev_stage, by which
-// time they have finished copying rows out of its planes.
-static int csf_step_group(lbm_domain* const* ds, int n, int n_steps)
+// linked two-phase slabs in lock step (lbm_step_group)
+int tp_step_group(lbm_domain* const* ds, int n, int n_steps)
 {
-  auto on = [](lbm_domain* d) { return cudaSetDevice(d->cfg.device); };
-  auto wait_neighbours = [&](lbm_domain* d, cudaEvent_t lbm_domain::*ev) -> int {
-    for (lbm_domain* o : {d->link_lo, d->link_hi})
-      if (o && o != d) LBM_CUDA(cudaStreamWaitEvent(d->stream, o->*ev, 0));
-    return LBM_OK;
-  };
+  const TpStage& first = tp_schedule(ds, n).stage[0];
   for (int i = 0; i < n; i++)
   {
     LBM_CUDA(on(ds[i]));
     LBM_CUDA(cudaEventRecord(ds[i]->ev_begin, ds[i]->stream));
+    if (first.wait) LBM_CUDA(cudaEventRecord(ds[i]->*first.wait, ds[i]->stream));  // MRTCG / RK: "nobody is reading my planes"
   }
   for (int s = 0; s < n_steps; s++)
   {
-    bool fuse = true;  // all slabs or none: the halo rows a slab sends must be the ones its neighbour's stage expects
-    for (int i = 0; i < n; i++) fuse = fuse && csf_can_fuse(ds[i]);
-    for (int i = 0; i < n; i++)
-    {
-      LBM_CUDA(on(ds[i]));
-      LBM_TRY(fuse ? csf_fused_moments(ds[i]) : csf_phase_moments(ds[i]));
-      LBM_CUDA(cudaEventRecord(ds[i]->ev_ready, ds[i]->stream));
-    }
-    for (int i = 0; i < n; i++)
-    {
-      LBM_CUDA(on(ds[i]));
-      LBM_TRY(wait_neighbours(ds[i], &lbm_domain::ev_ready));
-      LBM_TRY(tp_link_halo_planes(ds[i], &TwoPhaseState::mom, M_COUNT));
-      LBM_TRY(fuse ? csf_fused_normals(ds[i]) : csf_phase_normals(ds[i]));
-      LBM_CUDA(cudaEventRecord(ds[i]->ev_packet, ds[i]->stream));
-    }
-    for (int i = 0; i < n; i++)
-    {
-      LBM_CUDA(on(ds[i]));
-      LBM_TRY(wait_neighbours(ds[i], &lbm_domain::ev_packet));
-      LBM_TRY(tp_link_halo_planes(ds[i], &TwoPhaseState::aux, 2));
-      LBM_TRY(fuse ? csf_fused_collide(ds[i]) : csf_phase_collide(ds[i]));
-      LBM_CUDA(cudaEventRecord(ds[i]->ev_stage, ds[i]->stream));
-    }
-    if (fuse)
+    const TpSchedule& sc = tp_schedule(ds, n);
+    for (const TpStage& st : sc.stage)
+      for (int i = 0; i < n; i++)
+      {
+        lbm_domain* d = ds[i];
+        LBM_CUDA(on(d));
+        if (st.wait) LBM_TRY(wait_linked(d, d->stream, st.wait));
+        if (st.halo) LBM_TRY(tp_link_halo_planes(d, st.halo, st.nplanes));
+        if (st.phase) LBM_TRY(st.phase(d));
+        LBM_CUDA(cudaEventRecord(d->*st.done, d->stream));
+      }
+    if (sc.swap_aux)
       for (int i = 0; i < n; i++) csf_fused_swap(ds[i]);
     for (int i = 0; i < n; i++)
     {
       lbm_domain* d = ds[i];
       LBM_CUDA(on(d));
-      LBM_TRY(wait_neighbours(d, &lbm_domain::ev_stage));
+      LBM_TRY(wait_linked(d, d->stream, &lbm_domain::ev_stage));
       ProfScope ps(d, LBM_PROF_GHOST);
       if (d->link_lo || d->link_hi) LBM_TRY(link_exchange(d, d->cur, d->stream));
       else LBM_TRY(wrap_ghost_rows_local(d, d->cur, d->stream));
@@ -2921,6 +2755,72 @@ static int csf_step_group(lbm_domain* const* ds, int n, int n_steps)
     LBM_CUDA(on(ds[i]));
     LBM_CUDA(cudaEventRecord(ds[i]->ev_end, ds[i]->stream));
   }
+  return LBM_OK;
+}
+
+// (here, below both kernel tables: the switches are read once, and every table entry gets its attributes)
+int tp_create(lbm_domain* d)
+{
+  TwoPhaseState* tp = new TwoPhaseState();
+  d->tp = tp;
+  tp->model = d->cfg.model == LBM_MODEL_MRTCG ? TP_MRTCG : (d->cfg.model == LBM_MODEL_MRT_CSF ? TP_CSF : TP_RK);
+  tp->mg.pm = ((d->g.Y + 4 + 15) / 16) * 16;
+  tp->mg.mplane = (long long)(d->g.Xl + 4) * tp->mg.pm;
+  const size_t bytes = sizeof(double) * M_COUNT * tp->mg.mplane;
+  LBM_CUDA(cudaMalloc(&tp->mom, bytes));
+  LBM_CUDA(cudaMemset(tp->mom, 0, bytes));
+  TpParams& p = tp->p;
+  const lbm_config& c = d->cfg;
+  if (!(c.red.rho_0 > 0.0) || !(c.blue.rho_0 > 0.0) || !(c.delta > 0.0))
+  {
+    set_error("two-phase model: red/blue initial_density and delta must be positive");
+    return LBM_ERR_INVALID;
+  }
+  tp_fill_params(c, (TpModel)tp->model, p);
+  if (tp->model == TP_CSF)
+  {
+    const size_t ab = sizeof(double) * 4 * tp->mg.mplane;
+    LBM_CUDA(cudaMalloc(&tp->aux, ab));
+    LBM_CUDA(cudaMemset(tp->aux, 0, ab));
+    int staged = 2;
+    bool pipe = false;
+    if (const char* e = getenv("LBM_CSF_FUSED")) tp->csf_fused = atoi(e) != 0;
+    if (const char* e = getenv("LBM_CSF_PIPE")) pipe = atoi(e) != 0;
+    if (const char* e = getenv("LBM_CSF_STAGED")) staged = atoi(e);
+    tp->csf_kernel = csf_pick_kernel(staged, pipe);
+    if (tp->csf_fused)
+    {
+      LBM_CUDA(cudaMalloc(&tp->aux_next, ab));
+      LBM_CUDA(cudaMemset(tp->aux_next, 0, ab));
+    }
+  }
+  else
+  {
+    // MRTCG (H = 2): the stash frees shared memory for a third block per SM (+17 %).  RK (H = 1) runs two blocks either way
+    // and is 1 % faster with its two resident rows left in the stage slots
+    bool pipe = true, staged = true, stash = tp->model == TP_MRTCG;
+    int stages = 0;
+    if (const char* e = getenv("LBM_TP_PIPE")) pipe = atoi(e) != 0;
+    if (const char* e = getenv("LBM_TP_STAGED")) staged = atoi(e) != 0;
+    if (const char* e = getenv("LBM_TP_NS")) stages = atoi(e);
+    if (const char* e = getenv("LBM_TP_STASH")) stash = atoi(e) != 0;
+    tp->kernel = tp_pick_kernel(tp->model, staged, stash, stages, pipe);
+  }
+  // every instantiation a switch can select, whichever this domain runs
+  auto set_attributes = [](const auto& table) -> int {
+    for (const auto& k : table)
+    {
+      LBM_CUDA(cudaFuncSetAttribute(k.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem));
+      if (k.staged) LBM_CUDA(cudaFuncSetAttribute(k.kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    }
+    return LBM_OK;
+  };
+  LBM_TRY(set_attributes(tp_kernels));
+  LBM_TRY(set_attributes(csf_kernels));
+  LBM_CUDA(cudaFuncSetAttribute(k_csf_collide_ring<MODE_LOCAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CsfRing::SMEM));
+  LBM_CUDA(cudaFuncSetAttribute(k_csf_collide_ring<MODE_PULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CsfRing::SMEM));
+  if (const char* e = getenv("LBM_TP_RPB")) tp->rpb_override = atoi(e);
+  if (const char* e = getenv("LBM_TP_OVERLAP")) tp->ring_overlap = atoi(e) != 0;  // (off by default: see tp_steps_ring)
   return LBM_OK;
 }
 
@@ -3186,10 +3086,10 @@ int lbm_init_two_phase(lbm_domain* d, const double* rho_r, const double* rho_b, 
   LBM_CUDA(cudaMemcpyAsync(tmp + N, rho_b, sizeof(double) * N, cudaMemcpyHostToDevice, d->stream));
   LBM_CUDA(cudaMemcpyAsync(tmp + 2 * N, u, sizeof(double) * 2 * N, cudaMemcpyHostToDevice, d->stream));
   if (d->tp->aux) LBM_CUDA(cudaMemsetAsync(d->tp->aux, 0, sizeof(double) * 4 * d->tp->mg.mplane, d->stream));
-  if (d->tp->model != TP_RK)
-    k_tp_init<TP_MRTCG><<<cdiv(N, 256), 256, 0, d->stream>>>(d->buf[0][d->cur], d->buf[1][d->cur], d->g, d->tp->mg, d->tp->mom, d->tp->p, tmp, tmp + N, tmp + 2 * N);
-  else
-    k_tp_init<TP_RK><<<cdiv(N, 256), 256, 0, d->stream>>>(d->buf[0][d->cur], d->buf[1][d->cur], d->g, d->tp->mg, d->tp->mom, d->tp->p, tmp, tmp + N, tmp + 2 * N);
+  with_model(d->tp, [&](auto M) {
+    k_tp_init<M><<<cdiv(N, 256), 256, 0, d->stream>>>(d->buf[0][d->cur], d->buf[1][d->cur], d->g, d->tp->mg, d->tp->mom, d->tp->p, tmp, tmp + N, tmp + 2 * N);
+    return LBM_OK;
+  });
   d->launches++;
   int s = tp_pad(d);
   if (s == LBM_OK) s = comm_exchange_moments(d);

@@ -2,7 +2,6 @@
 
   kernel<targs><<<grid, block, smem, stream>>>(args)   ->  emu::launch(emu::LaunchCfg(grid, block, smem, stream), kernel<targs>, args)
   extern __shared__ T name[];                          ->  T* name = (T*)emu::dyn_smem();
-  asm volatile("ptx ..." ...);                         ->  ;          (only the optional L2-hint paths use inline PTX)
   #include <cuda_runtime.h>                            ->  #include "cuda_emu.hpp"
 
 Nothing else is touched: the kernels' bodies are compiled exactly as written.  usage: preprocess.py in.cu out.cpp"""
@@ -73,7 +72,6 @@ def main(src, dst):
     s = open(src).read()
     s = rewrite_launches(s)
     s = re.sub(r"extern\s+__shared__\s+(\w+)\s+(\w+)\[\];", r"\1* \2 = (\1*)emu::dyn_smem();", s)
-    s = re.sub(r"asm volatile\(.*?\);", ";", s)
     s = s.replace("#include <cuda_runtime.h>", '#include "cuda_emu.hpp"')
     with open(dst, "w") as f:
         f.write(f'#line 1 "{src}"\n' + s)
