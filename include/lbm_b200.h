@@ -298,6 +298,33 @@ int lbm_body_force_read(lbm_domain* d, double* F, int max_steps, int* n_steps, l
 int lbm_body_force_stop(lbm_domain* d);
 
 /* ------------------------------------------------------------------------------------------------
+ * Time-averaged fields, accumulated on the device inside the step — replaces averaging the rho / u snapshots that the
+ * reference's drivers torch::save for offline post-processing (mean wake, mean pressure rho / 3, Reynolds stresses).
+ * The step kernels fold the moments their collision uses into per-node Welford accumulators (mean_rho, mean_ux, mean_uy,
+ * Mxx, Myy, Mxy, fp64): a sampled step reads and writes 96 B/node more, an unsampled one nothing.
+ *   - the moments of a step are those lbm_get_moments returns for the state the step starts from (KBC after
+ *     lbm_set_moments: the moments given); a sampled step updates every node of the slab exactly once
+ *   - the record keeps running across lbm_bc_commit (the new listed nodes are sampled by the new rules), across imports
+ *     (lbm_set_f, lbm_init_equilibrium: the next step samples the imported state) and across lbm_use_graph on / off (the
+ *     sample counter lives on the device, so replayed step pairs sample the right steps)
+ *   - linked slabs (lbm_step_group), NCCL ring ranks and bound blocks each accumulate their own rows with no
+ *     communication; the global fields are the slabs' fields stacked along axis 0
+ * Single-phase models only: LBM_MODEL_BGK (any equilibrium and force), LBM_MODEL_KBC, LBM_MODEL_BGK_ADE (fluid lattice).
+ * Two-phase models: LBM_ERR_UNSUPPORTED.  Without a record the step launches exactly the kernels it did before.
+ * ---------------------------------------------------------------------------------------------- */
+/* start (or restart) accumulating statistics of the moments each step's collision uses — the values lbm_get_moments
+ * returns for the state the step starts from (KBC after lbm_set_moments: the moments given).  Step k after the call
+ * (k = 0, 1, ...) is a sample when k % every == 0.  Each domain accumulates its own rows; nothing crosses to the host.
+ * every < 1: LBM_ERR_INVALID.  Calling it again discards what was accumulated and restarts from n = 0.                   */
+int lbm_stats_start(lbm_domain* d, int every);
+/* rho_mean {Xl,Y,1}, u_mean {Xl,Y,2}, u_cov {Xl,Y,3} = (<u'u'>, <v'v'>, <u'v'>), divided by n (not n-1); any may be NULL.
+ * *n_samples = n, the samples taken so far; with n = 0 the buffers are left untouched.  No record: LBM_ERR_INVALID.
+ * Synchronises the domain's stream.                                                                                        */
+int lbm_stats_read(lbm_domain* d, double* rho_mean, double* u_mean, double* u_cov, long long* n_samples);
+/* end the record and free its accumulators (no record: LBM_ERR_INVALID) */
+int lbm_stats_stop(lbm_domain* d);
+
+/* ------------------------------------------------------------------------------------------------
  * Time stepping — replaces the loop body of each driver (SURVEY §3.1-3.3)
  * ---------------------------------------------------------------------------------------------- */
 /* advance n_steps; asynchronous on the domain's stream */

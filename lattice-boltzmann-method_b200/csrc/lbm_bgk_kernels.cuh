@@ -17,6 +17,9 @@
 //                     on the same stream and overwrites what that wrote for listed nodes.
 //   k_fix_copy, k_pressure_pack/apply : pre-stream rules applied to the freshly written f_coll
 //                     (zero-gradient copies, pressure-periodic rows).
+//   k_bgk_interior_stats / k_bgk_boundary_stats : the same two kernels (STATS = true of their bodies bgk_interior /
+//                     bgk_boundary) while a statistics record is on (lbm_stats_start): they also fold the moments their
+//                     collision uses into the Welford accumulators of the time-averaged fields.
 #pragma once
 #include "lbm_device.cuh"
 
@@ -60,6 +63,56 @@ struct FixEntry
   int lattice;
   int pad;
 };
+
+// ------------------------------------------------------------------------------------------------
+// time-averaged moments (lbm_stats_start)
+// ------------------------------------------------------------------------------------------------
+// Six planes of Xl x pitch doubles, node (x, y) at x * pitch + y: the running means of rho, ux, uy, then the Welford sums
+// Mxx, Myy, Mxy of the products of the deviations.  Sample k (n = k + 1) updates them in an order NumPy restates,
+//   d = v - mean;  mean += d * (1 / n);  M_ab += d_a * (v_b - mean_b)
+// (raw sums of u^2 would lose the fluctuation's digits next to a steady mean).  1 / n is rounded once per step by
+// k_stats_tick: an fp64 division in the step kernels would call its slow-path subroutine three times per node, and the
+// calls cost the listed-node kernel a stack frame.  Every node is updated by exactly one launch of a step: listed nodes by
+// k_bgk_boundary, every other node by k_bgk_interior.
+struct StatsClock
+{
+  long long count;  // steps since lbm_stats_start
+  double inv_n;     // 1 / n of this step's sample, 0 when the step is no sample
+};
+
+struct StatsArgs
+{
+  double* acc;              // plane k at acc + k * plane
+  long long plane;          // Xl * pitch
+  const StatsClock* clock;  // k_stats_tick advances it after all three launches of a step
+  int words;                // 32-bit words per row of `listed`
+  const unsigned* listed;   // early rows only: bit y of row x is set when (x, y) is a listed node; nullptr otherwise
+};
+
+// a = (mean rho, mean ux, mean uy, Mxx, Myy, Mxy) of one node
+__device__ __forceinline__ void welford(double (&a)[6], double inv_n, double rho, double ux, double uy)
+{
+  const double dr = rho - a[0];
+  a[0] = a[0] + dr * inv_n;
+  const double dx = ux - a[1];
+  a[1] = a[1] + dx * inv_n;
+  const double dy = uy - a[2];
+  a[2] = a[2] + dy * inv_n;
+  a[3] = a[3] + dx * (ux - a[1]);
+  a[4] = a[4] + dy * (uy - a[2]);
+  a[5] = a[5] + dx * (uy - a[2]);
+}
+
+// one node (listed-node kernel)
+__device__ __forceinline__ void stats_node(const StatsArgs& s, double inv_n, long long i, double rho, double ux, double uy)
+{
+  double a[6];
+#pragma unroll
+  for (int k = 0; k < 6; k++) a[k] = s.acc[k * s.plane + i];
+  welford(a, inv_n, rho, ux, uy);
+#pragma unroll
+  for (int k = 0; k < 6; k++) s.acc[k * s.plane + i] = a[k];
+}
 
 // ------------------------------------------------------------------------------------------------
 // interior kernel
@@ -153,12 +206,13 @@ __device__ __forceinline__ void load_streamed_pair(const double* __restrict__ ba
 // kernel grow from 76 to 126 registers and cost the cylinder workload 8 %.  For the KBC instantiation (126 registers,
 // 4 blocks/SM) forcing more resident blocks was measured at 8192^2: 5 blocks (spills 224 B) 31.4 GLUPS, 6 (404 B) 24.8,
 // 8 (608 B) 18.4, against 35.9 as compiled here — that collision needs its registers.
-template <int MODE, int EQ, int FORCE, bool ADE>
-__global__ void __launch_bounds__(128)
-k_bgk_interior(const double* __restrict__ fsrc, double* __restrict__ fdst, const double* __restrict__ gsrc,
-               double* __restrict__ gdst, const SlabGeom g, const BgkParams p, const int* __restrict__ rows, int npairs,
-               double* __restrict__ out_f, double* __restrict__ out_g)
+template <int MODE, int EQ, int FORCE, bool ADE, bool STATS>
+__device__ __forceinline__ void
+bgk_interior(const double* __restrict__ fsrc, double* __restrict__ fdst, const double* __restrict__ gsrc,
+             double* __restrict__ gdst, const SlabGeom g, const BgkParams p, const int* __restrict__ rows, int npairs,
+             double* __restrict__ out_f, double* __restrict__ out_g, const StatsArgs st)
 {
+  static_assert(!(STATS && MODE == MODE_PULL_ONLY), "a pull-only pass is no step: nothing to sample");
   const int pi = blockIdx.x * blockDim.x + threadIdx.x;
   const int x = rows[blockIdx.y];
   const int lane = threadIdx.x & 31;
@@ -261,6 +315,39 @@ k_bgk_interior(const double* __restrict__ fsrc, double* __restrict__ fdst, const
 #pragma unroll
       for (int q = 0; q < 9; q++) st_pair(fdst + q * g.plane + o, fa[q], fb[q]);
     }
+    if constexpr (STATS)
+    {
+      const double inv_n = st.clock->inv_n;
+      if (active && inv_n != 0.0)
+      {
+        // a listed node of an early row: k_bgk_boundary overwrites this collision and samples the node itself
+        bool skip_a = false, skip_b = false;
+        if (st.listed != nullptr)
+        {
+          const unsigned w = st.listed[(long long)x * st.words + (y >> 5)];  // y even: y and y + 1 share the word
+          skip_a = (w >> (y & 31)) & 1u;
+          skip_b = (w >> ((y + 1) & 31)) & 1u;
+        }
+        double* ps = st.acc + (o - g.pitch);  // (x, y) at x * pitch + y
+        double a[6], b[6];
+#pragma unroll
+        for (int k = 0; k < 6; k++)
+        {
+          const double2 v = *reinterpret_cast<const double2*>(ps + k * st.plane);  // (read and written here: no __ldg)
+          a[k] = v.x;
+          b[k] = v.y;
+        }
+        welford(a, inv_n, rho_a, ux_a, uy_a);
+        welford(b, inv_n, rho_b, ux_b, uy_b);
+#pragma unroll
+        for (int k = 0; k < 6; k++)
+        {
+          if (!skip_a && !skip_b) st_pair(ps + k * st.plane, a[k], b[k]);
+          else if (!skip_a) ps[k * st.plane] = a[k];
+          else if (!skip_b) ps[k * st.plane + 1] = b[k];
+        }
+      }
+    }
     if constexpr (ADE)
     {
       double ga[9], gb[9];
@@ -277,15 +364,36 @@ k_bgk_interior(const double* __restrict__ fsrc, double* __restrict__ fdst, const
   }
 }
 
+template <int MODE, int EQ, int FORCE, bool ADE>
+__global__ void __launch_bounds__(128)
+k_bgk_interior(const double* __restrict__ fsrc, double* __restrict__ fdst, const double* __restrict__ gsrc,
+               double* __restrict__ gdst, const SlabGeom g, const BgkParams p, const int* __restrict__ rows, int npairs,
+               double* __restrict__ out_f, double* __restrict__ out_g)
+{
+  bgk_interior<MODE, EQ, FORCE, ADE, false>(fsrc, fdst, gsrc, gdst, g, p, rows, npairs, out_f, out_g, StatsArgs{});
+}
+
+// the step with a statistics record on (lbm_stats_start): an entry point of its own, so that the kernels without a record
+// keep their names, parameters and machine code
+template <int MODE, int EQ, int FORCE, bool ADE>
+__global__ void __launch_bounds__(128)
+k_bgk_interior_stats(const double* __restrict__ fsrc, double* __restrict__ fdst, const double* __restrict__ gsrc,
+                     double* __restrict__ gdst, const SlabGeom g, const BgkParams p, const int* __restrict__ rows, int npairs,
+                     const StatsArgs st)
+{
+  bgk_interior<MODE, EQ, FORCE, ADE, true>(fsrc, fdst, gsrc, gdst, g, p, rows, npairs, nullptr, nullptr, st);
+}
+
 // ------------------------------------------------------------------------------------------------
 // boundary kernel: one thread per listed node
 // ------------------------------------------------------------------------------------------------
-template <int MODE, int EQ, int FORCE, bool ADE>
-__global__ void __launch_bounds__(128)
-k_bgk_boundary(const double* __restrict__ fsrc, double* __restrict__ fdst, const double* __restrict__ gsrc,
-               double* __restrict__ gdst, const SlabGeom g, const BgkParams p, const BoundaryTable t,
-               double* __restrict__ out_f, double* __restrict__ out_g)
+template <int MODE, int EQ, int FORCE, bool ADE, bool STATS>
+__device__ __forceinline__ void
+bgk_boundary(const double* __restrict__ fsrc, double* __restrict__ fdst, const double* __restrict__ gsrc,
+             double* __restrict__ gdst, const SlabGeom g, const BgkParams p, const BoundaryTable t,
+             double* __restrict__ out_f, double* __restrict__ out_g, const StatsArgs st)
 {
+  static_assert(!(STATS && MODE == MODE_PULL_ONLY), "a pull-only pass is no step: nothing to sample");
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= t.n) return;
   const int x = t.x[i], y = t.y[i];
@@ -419,6 +527,28 @@ k_bgk_boundary(const double* __restrict__ fsrc, double* __restrict__ fdst, const
     t.mom_cur[4 * i + 2] = uy;
     t.mom_cur[4 * i + 3] = C;
   }
+  if constexpr (STATS)
+  {
+    const double inv_n = st.clock->inv_n;
+    if (inv_n != 0.0) stats_node(st, inv_n, o - g.pitch, rho, ux, uy);  // (x, y) at x * pitch + y
+  }
+}
+
+template <int MODE, int EQ, int FORCE, bool ADE>
+__global__ void __launch_bounds__(128)
+k_bgk_boundary(const double* __restrict__ fsrc, double* __restrict__ fdst, const double* __restrict__ gsrc,
+               double* __restrict__ gdst, const SlabGeom g, const BgkParams p, const BoundaryTable t,
+               double* __restrict__ out_f, double* __restrict__ out_g)
+{
+  bgk_boundary<MODE, EQ, FORCE, ADE, false>(fsrc, fdst, gsrc, gdst, g, p, t, out_f, out_g, StatsArgs{});
+}
+
+template <int MODE, int EQ, int FORCE, bool ADE>
+__global__ void __launch_bounds__(128)
+k_bgk_boundary_stats(const double* __restrict__ fsrc, double* __restrict__ fdst, const double* __restrict__ gsrc,
+                     double* __restrict__ gdst, const SlabGeom g, const BgkParams p, const BoundaryTable t, const StatsArgs st)
+{
+  bgk_boundary<MODE, EQ, FORCE, ADE, true>(fsrc, fdst, gsrc, gdst, g, p, t, nullptr, nullptr, st);
 }
 
 // ------------------------------------------------------------------------------------------------

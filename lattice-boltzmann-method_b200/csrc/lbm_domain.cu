@@ -110,6 +110,7 @@ struct LaunchArgs
   double* snap_rho = nullptr;  // MODE_PULL_ONLY: write moments here instead of the AoS populations
   double* snap_u = nullptr;
   int prof_cls = LBM_PROF_INTERIOR;  // profiling class of the interior launch
+  bool early = false;  // the early rows of a step: with a statistics record, the interior kernel skips the listed nodes
 };
 
 // Threads per block of the side chain's kernels (listed nodes, stages, ghost rows).  (32-thread blocks, so that a pending
@@ -117,7 +118,7 @@ struct LaunchArgs
 // listed-node kernel takes 79 us beside the bulk launch of a 2700 x 2100 grid against 13 us alone either way.)
 constexpr int SIDE_NT = 128;
 
-template <int MODE, int EQ, int FORCE, bool ADE>
+template <int MODE, int EQ, int FORCE, bool ADE, bool STATS>
 static int launch_bgk(lbm_domain* d, const LaunchArgs& a)
 {
   BgkParams p;
@@ -137,6 +138,15 @@ static int launch_bgk(lbm_domain* d, const LaunchArgs& a)
   p.Y = d->g.Y;
   p.snap_rho = a.snap_rho;
   p.snap_u = a.snap_u;
+  StatsArgs st{};  // (STATS = false: unused)
+  if constexpr (STATS)
+  {
+    st.acc = d->st.d_acc;
+    st.plane = (long long)d->g.Xl * d->g.pitch;
+    st.clock = d->st.d_clock;
+    st.words = d->st.words;
+    st.listed = a.early ? d->st.d_listed : nullptr;
+  }
   if (a.rows && d->npairs > 0 && a.n_rows > 0)
   {
     ProfScope ps(d, a.prof_cls, a.stream);
@@ -146,8 +156,12 @@ static int launch_bgk(lbm_domain* d, const LaunchArgs& a)
     for (int c : {96, 64})
       if ((long long)cdiv(d->npairs, c) * c < (long long)cdiv(d->npairs, bs) * bs) bs = c;
     dim3 grid(cdiv(d->npairs, bs), a.n_rows);
-    k_bgk_interior<MODE, EQ, FORCE, ADE><<<grid, bs, 0, a.stream>>>(d->buf[0][a.s], d->buf[0][a.t], d->buf[1][a.s], d->buf[1][a.t],
-                                                                    d->g, p, a.rows, d->npairs, d->d_aos[0], d->d_aos[1]);
+    if constexpr (STATS)
+      k_bgk_interior_stats<MODE, EQ, FORCE, ADE><<<grid, bs, 0, a.stream>>>(d->buf[0][a.s], d->buf[0][a.t], d->buf[1][a.s], d->buf[1][a.t],
+                                                                            d->g, p, a.rows, d->npairs, st);
+    else
+      k_bgk_interior<MODE, EQ, FORCE, ADE><<<grid, bs, 0, a.stream>>>(d->buf[0][a.s], d->buf[0][a.t], d->buf[1][a.s], d->buf[1][a.t],
+                                                                      d->g, p, a.rows, d->npairs, d->d_aos[0], d->d_aos[1]);
     d->launches++;
   }
   if (a.listed && d->nb > 0)
@@ -160,15 +174,19 @@ static int launch_bgk(lbm_domain* d, const LaunchArgs& a)
     bt.ent = d->d_ent;
     bt.mom_prev = d->d_mom[d->mom_cur];
     bt.mom_cur = MODE == MODE_PULL_ONLY ? nullptr : d->d_mom[d->mom_cur ^ 1];
-    k_bgk_boundary<MODE, EQ, FORCE, ADE><<<cdiv(d->nb, SIDE_NT), SIDE_NT, 0, a.stream>>>(d->buf[0][a.s], d->buf[0][a.t], d->buf[1][a.s],
-                                                                                d->buf[1][a.t], d->g, p, bt, d->d_aos[0], d->d_aos[1]);
+    if constexpr (STATS)
+      k_bgk_boundary_stats<MODE, EQ, FORCE, ADE><<<cdiv(d->nb, SIDE_NT), SIDE_NT, 0, a.stream>>>(d->buf[0][a.s], d->buf[0][a.t], d->buf[1][a.s],
+                                                                                          d->buf[1][a.t], d->g, p, bt, st);
+    else
+      k_bgk_boundary<MODE, EQ, FORCE, ADE><<<cdiv(d->nb, SIDE_NT), SIDE_NT, 0, a.stream>>>(d->buf[0][a.s], d->buf[0][a.t], d->buf[1][a.s],
+                                                                                  d->buf[1][a.t], d->g, p, bt, d->d_aos[0], d->d_aos[1]);
     d->launches++;
   }
   LBM_CUDA(cudaGetLastError());
   return LBM_OK;
 }
 
-template <int MODE>
+template <int MODE, bool STATS = false>
 static int dispatch_bgk(lbm_domain* d, const LaunchArgs& a)
 {
   const bool ade = d->cfg.model == LBM_MODEL_BGK_ADE;
@@ -177,12 +195,12 @@ static int dispatch_bgk(lbm_domain* d, const LaunchArgs& a)
   {
     // with an immersed body (BASELINE configs[4] "with immersed-boundary coupling"): the cylinder driver's force term on the
     // fluid lattice, the ADE lattice advected by the same u
-    if (fo == FORCE_IBM) return launch_bgk<MODE, EQ_COMP, FORCE_IBM, true>(d, a);
-    return launch_bgk<MODE, EQ_COMP, FORCE_NONE, true>(d, a);
+    if (fo == FORCE_IBM) return launch_bgk<MODE, EQ_COMP, FORCE_IBM, true, STATS>(d, a);
+    return launch_bgk<MODE, EQ_COMP, FORCE_NONE, true, STATS>(d, a);
   }
-  if (d->cfg.model == LBM_MODEL_KBC) return launch_bgk<MODE, EQ_KBC, FORCE_NONE, false>(d, a);
+  if (d->cfg.model == LBM_MODEL_KBC) return launch_bgk<MODE, EQ_KBC, FORCE_NONE, false, STATS>(d, a);
 #define LBM_CASE(E, F) \
-  if (eq == E && fo == F) return launch_bgk<MODE, E, F, false>(d, a);
+  if (eq == E && fo == F) return launch_bgk<MODE, E, F, false, STATS>(d, a);
   LBM_CASE(EQ_COMP, FORCE_NONE)
   LBM_CASE(EQ_COMP, FORCE_UNIFORM)
   LBM_CASE(EQ_COMP, FORCE_IBM)
@@ -196,8 +214,11 @@ static int dispatch_bgk(lbm_domain* d, const LaunchArgs& a)
   return LBM_ERR_INVALID;
 }
 
+// a step's launches: with a statistics record on, the STATS instantiations
 static int dispatch_mode(lbm_domain* d, int mode, const LaunchArgs& a)
 {
+  if (d->st.on && mode == MODE_LOCAL) return dispatch_bgk<MODE_LOCAL, true>(d, a);
+  if (d->st.on && mode == MODE_PULL) return dispatch_bgk<MODE_PULL, true>(d, a);
   if (mode == MODE_LOCAL) return dispatch_bgk<MODE_LOCAL>(d, a);
   if (mode == MODE_PULL) return dispatch_bgk<MODE_PULL>(d, a);
   return dispatch_bgk<MODE_PULL_ONLY>(d, a);
@@ -303,10 +324,12 @@ int step_early(lbm_domain* d)
     LBM_CUDA(cudaStreamWaitEvent(d->side, d->ev_early, 0));
     LaunchArgs a{d->cur, d->cur ^ 1, d->d_rows_early, d->n_early, false, d->ibm.next_slot, d->side};
     a.prof_cls = LBM_PROF_EARLY;
+    a.early = true;
     return dispatch_mode(d, mode, a);
   }
   LaunchArgs a{d->cur, d->cur ^ 1, d->d_rows_early, d->n_early, false, d->ibm.next_slot, d->stream};
   a.prof_cls = LBM_PROF_EARLY;
+  a.early = true;
   LBM_TRY(dispatch_mode(d, mode, a));
   LBM_CUDA(cudaEventRecord(d->ev_early, d->stream));
   return LBM_OK;
@@ -405,6 +428,7 @@ int step_bulk(lbm_domain* d)
   const int mode = d->post_stream ? MODE_LOCAL : MODE_PULL;
   LaunchArgs a{d->cur, d->cur ^ 1, d->d_rows_bulk, d->n_bulk, false, d->ibm.next_slot, d->stream};
   LBM_TRY(dispatch_mode(d, mode, a));
+  LBM_TRY(stats_tick(d));
   d->cur ^= 1;
   d->mom_cur ^= 1;
   d->post_stream = false;
@@ -826,6 +850,7 @@ int commit_boundary_tables(lbm_domain* d)
   }
   d->rows_dirty = true;
   d->side_ready = false;
+  if (d->st.on) LBM_TRY(stats_listed_mask(d));
 
   // ---- upload
   d->nb = nb;
@@ -1061,6 +1086,7 @@ int lbm_destroy(lbm_domain* d)
   if (d->stream) cudaStreamSynchronize(d->stream);
   if (d->side) cudaStreamSynchronize(d->side);
   release_compiled(d);
+  stats_release(d);
   faces_release(d);
   ibm_release(d);
   tp_destroy(d);
@@ -1495,3 +1521,5 @@ int lbm_decompose_rows(int X, int n_ranks, int rank, int* x0, int* x1)
 
 // lbm_body_force_record / _read / _stop and their kernels
 #include "lbm_body_force.cuh"
+// lbm_stats_start / _read / _stop and their kernels
+#include "lbm_stats.cuh"

@@ -110,6 +110,18 @@ struct BodyForce
   long long* d_count = nullptr;   // steps recorded so far (advanced by the kernel, so graph replays count too)
 };
 
+// lbm_stats_start: time-averaged moments, accumulated by the STATS instantiations of the step kernels (lbm_stats.cuh)
+struct Stats
+{
+  bool on = false;
+  int every = 1;
+  double* d_acc = nullptr;       // [6][Xl][pitch]: mean rho, mean ux, mean uy, Mxx, Myy, Mxy (StatsArgs)
+  StatsClock* d_clock = nullptr; // steps since lbm_stats_start and 1 / n of the next sample (advanced on the device, so
+                                 // graph replays count too)
+  unsigned* d_listed = nullptr;  // [Xl][words]: one bit per listed node in an interior column, rebuilt by lbm_bc_commit
+  int words = 0;
+};
+
 struct ProfRec
 {
   cudaEvent_t a, b;
@@ -212,6 +224,7 @@ struct lbm_domain
   lbm::IbmState ibm;
   lbm::IbmGiven ibm_given;
   lbm::BodyForce bf;
+  lbm::Stats st;
   double ics2 = 1.0 / 3.0, ics4 = 1.0 / 9.0;  // source-term constants (lbm_set_force_region overrides them)
   // column-face bindings to other blocks (lbm_link_face): the populations entering through an edge column are read
   // from a tail appended to every lattice buffer, [side][3 populations][Xl] behind the nine planes
@@ -282,6 +295,10 @@ int faces_release(lbm_domain* d);                      // NCCL: ROI row segments
 // lbm_body_force.cuh (compiled inside lbm_domain.cu)
 void body_force_release(lbm_domain* d);
 int body_force_step(lbm_domain* d);  // side: the force of the step being enqueued into the ring (no-op when not recording)
+// lbm_stats.cuh (compiled inside lbm_domain.cu)
+void stats_release(lbm_domain* d);
+int stats_listed_mask(lbm_domain* d);  // (re)build the listed-node bit mask from listed_ids
+int stats_tick(lbm_domain* d);         // main, after the bulk rows: wait for the side chain, advance the sample counter
 // lbm_two_phase.cu
 int tp_create(lbm_domain* d);
 int tp_destroy(lbm_domain* d);

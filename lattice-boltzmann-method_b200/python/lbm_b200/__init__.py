@@ -107,6 +107,7 @@ EXPORTS = [
     "lbm_profile_enable", "lbm_profile_read", "lbm_step_group", "lbm_save_pt", "lbm_snapshot_async", "lbm_snapshot_wait", "lbm_set_moments", "lbm_get_interfacial_tension", "lbm_link_face", "lbm_set_force_region",
     "lbm_rk_diagnostics", "lbm_comm_check", "lbm_comm_share", "lbm_row_split", "lbm_comm_init_blocks", "lbm_link_face_rank", "lbm_comm_faces_commit",
     "lbm_body_force_record", "lbm_body_force_read", "lbm_body_force_stop",
+    "lbm_stats_start", "lbm_stats_read", "lbm_stats_stop",
 ]
 PROF_INTERIOR, PROF_BOUNDARY, PROF_FIXUP, PROF_GHOST, PROF_IBM, PROF_MOMENTS, PROF_EARLY = range(7)
 
@@ -151,6 +152,9 @@ def load():
         _lib.lbm_body_force_record.argtypes = [C.c_void_p, C.POINTER(C.c_ubyte), C.c_int, C.c_int, C.c_int]
         _lib.lbm_body_force_read.argtypes = [C.c_void_p, dp, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_longlong)]
         _lib.lbm_body_force_stop.argtypes = [C.c_void_p]
+        _lib.lbm_stats_start.argtypes = [C.c_void_p, C.c_int]
+        _lib.lbm_stats_read.argtypes = [C.c_void_p, dp, dp, dp, C.POINTER(C.c_longlong)]
+        _lib.lbm_stats_stop.argtypes = [C.c_void_p]
         _lib.lbm_step.argtypes = [C.c_void_p, C.c_int]
         _lib.lbm_last_step_ms.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
         _lib.lbm_kernel_launches.argtypes = [C.c_void_p, C.POINTER(C.c_longlong)]
@@ -431,6 +435,25 @@ class Domain:
     def body_force_stop(self):
         _chk(self.lib.lbm_body_force_stop(self.h))
         self._bf_capacity = 0
+
+    # ---- time-averaged fields, accumulated on the device inside the step
+    def stats_start(self, every=1):
+        """start (or restart) accumulating the mean and covariance of the moments each step's collision uses; step k after
+        the call is a sample when k % every == 0"""
+        _chk(self.lib.lbm_stats_start(self.h, int(every)))
+
+    def stats(self):
+        """(n, rho_mean {Xl,Y,1}, u_mean {Xl,Y,2}, u_cov {Xl,Y,3}): n samples so far, u_cov = (<u'u'>, <v'v'>, <u'v'>)
+        divided by n.  With n = 0 the three arrays are None.  Synchronises the domain."""
+        rho = np.empty((self.Xl, self.Y, 1)); u = np.empty((self.Xl, self.Y, 2)); cov = np.empty((self.Xl, self.Y, 3))
+        n = C.c_longlong()
+        _chk(self.lib.lbm_stats_read(self.h, rho.ctypes.data_as(dp), u.ctypes.data_as(dp), cov.ctypes.data_as(dp), C.byref(n)))
+        if n.value == 0:
+            return 0, None, None, None
+        return n.value, rho, u, cov
+
+    def stats_stop(self):
+        _chk(self.lib.lbm_stats_stop(self.h))
 
     # ---- stepping
     def step(self, n=1):
