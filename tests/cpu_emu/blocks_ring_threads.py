@@ -31,14 +31,16 @@ def main(Ln=64, steps=45):
     dom = cases.loop_blocks(Ln, omega)
     for k in cases.LOOP_BLOCKS:
         dom[k].set_f(f0[k])
+        dom[k].stats_start(3)
     L.step_group([dom[k] for k in cases.LOOP_BLOCKS], steps)
     want = {k: dom[k].get_f() for k in cases.LOOP_BLOCKS}
+    want_stats = {k: dom[k].stats() for k in cases.LOOP_BLOCKS}
     for d in dom.values():
         d.close()
     # four "processes"
     sync = threading.Barrier(4)
     shared = {"id": None}
-    got, errors = {}, []
+    got, got_stats, errors = {}, {}, []
 
     def worker(rank):
         try:
@@ -50,10 +52,12 @@ def main(Ln=64, steps=45):
             d.bc_commit()
             k = cases.LOOP_BLOCKS[rank]
             d.set_f(f0[k])
+            d.stats_start(3)  # each rank accumulates its own block
             d.step(steps // 2)
             mid = d.get_f()          # an export in the middle: the next step re-prepares the state (face tails of the current buffers)
             d.step(steps - steps // 2)
             got[k] = d.get_f()
+            got_stats[k] = d.stats()
             assert np.isfinite(mid).all()
             sync.wait()
             d.close()
@@ -69,7 +73,10 @@ def main(Ln=64, steps=45):
     ok = not errors and all(np.array_equal(got[k], want[k]) for k in cases.LOOP_BLOCKS)
     print("errors:", errors)
     print("blocks across ranks: bit-exact vs linked blocks =", ok)
-    return 0 if ok else 1
+    ok_stats = not errors and all(got_stats[k][0] == want_stats[k][0] == 15 and
+                                  all(np.array_equal(a, b) for a, b in zip(got_stats[k][1:], want_stats[k][1:])) for k in cases.LOOP_BLOCKS)
+    print("blocks across ranks: statistics record bit-exact vs linked blocks =", ok_stats)
+    return 0 if ok and ok_stats else 1
 
 
 if __name__ == "__main__":

@@ -78,6 +78,28 @@ def run_checks(rank, world, local, fresh_id, gather, barrier, extra=False):
             failures.append("poiseuille")
     d.close()
 
+    # ---- the statistics record on the ring: each rank accumulates its own rows, the pressure rows on the end ranks
+    d = L.Domain(L.default_config(x0=x0, x1=x1, device=local, **kw))
+    d.comm_init(fresh_id(), world, rank)
+    d.preset_poiseuille(rho_in, rho_out)
+    d.set_f(f0[x0:x1])
+    d.stats_start(2)
+    d.step(37)
+    n, r, u, c = d.stats()
+    got = [gather(a) for a in (r, u, c)]
+    if rank == 0:
+        mono = L.Domain(L.default_config(device=local, **kw))
+        mono.preset_poiseuille(rho_in, rho_out)
+        mono.set_f(f0)
+        mono.stats_start(2)
+        mono.step(37)
+        want = mono.stats()
+        ok = n == want[0] == 19 and all(np.array_equal(a, b) for a, b in zip(got, want[1:]))
+        print(f"poiseuille statistics ring of {world}: bit-exact vs monolithic = {ok}")
+        if not ok:
+            failures.append("poiseuille-stats")
+    d.close()
+
     # ---- MRT colour gradient: population ghost rows + 2-row moment halos
     from oracle_lib import MrtcgParams, Oracle
 
@@ -225,18 +247,29 @@ def run_checks(rank, world, local, fresh_id, gather, barrier, extra=False):
     d.preset_free_stream(u_lb, 0.0)
     d.ibm_set_markers(xs, ys)
     d.set_f(g["f0"][x0:x1])
+    d.body_force_record(capacity=40)
     d.step(40)
     got = gather(d.get_f())
+    part, first = d.body_force()
+    parts = gather(part[None])
     if rank == 0:
         mono = L.Domain(L.default_config(device=local, **kw))
         mono.preset_free_stream(u_lb, 0.0)
         mono.ibm_set_markers(xs, ys)
         mono.set_f(g["f0"])
+        mono.body_force_record(capacity=40)
         mono.step(40)
         ok = np.array_equal(got, mono.get_f())
         print(f"cylinder across the cuts, ring of {world}: bit-exact vs monolithic = {ok}")
         if not ok:
             failures.append("cylinder-straddling")
+        # each rank sums the ROI nodes on its own rows: the parts add up to the whole in another order
+        F = mono.body_force()[0]
+        err = float(np.abs(parts.sum(axis=0) - F).max())
+        ok = first == 0 and parts.shape == (world, 40, 2) and np.abs(F).max() > 0 and err <= 1e-13 * np.abs(F).max()
+        print(f"cylinder body force across the cuts, ring of {world}: parts add up to the monolithic record = {ok} ({err:.1e})")
+        if not ok:
+            failures.append("cylinder-body-force")
     d.close()
 
     if extra:

@@ -55,15 +55,17 @@ def test_gpu_parity_tests_pass_on_the_emulated_device(emu_lib):
 def test_shared_memory_ring_kernels_do_not_depend_on_thread_order(emu_lib, order):
     """The threads of a block start and resume in reversed / shuffled order.  A missing barrier around the shared-memory
     rings of k_tp_fused / k_csf_collide_ring makes these runs fail (checked by deleting the ring's __syncthreads).  Every
-    instantiation of the two-phase step runs here too (test_gpu_tp_variants.py: stage slots, mbarrier parities, ring rows)."""
-    r = run_emulated(["tests/test_gpu_two_phase.py", "tests/test_gpu_csf.py", "tests/test_gpu_tp_variants.py"], 900, order)
+    instantiation of the two-phase step runs here too (test_gpu_tp_variants.py: stage slots, mbarrier parities, ring rows),
+    and both records' kernels (test_gpu_records_exact.py: the body-force block reductions, the statistics planes)."""
+    r = run_emulated(["tests/test_gpu_two_phase.py", "tests/test_gpu_csf.py", "tests/test_gpu_tp_variants.py",
+                      "tests/test_gpu_records_exact.py"], 1500, order)
     assert r.returncode == 0, r.stdout[-4000:]
 
 
 def test_kernels_under_address_sanitizer():
     """Device buffers are heap blocks of the emulated runtime: an out-of-bounds load or store of a kernel (or of the host
     code around it) is an AddressSanitizer report.  The two-phase and CSF tests here (ragged and tiny grids included, every
-    two-phase kernel instantiation at one-row bands); `make -C tests/cpu_emu SAN=1` + LBM_EMU_ASAN=1 runs any of the others the same way."""
+    two-phase kernel instantiation at one-row bands) and the records' tests; `make -C tests/cpu_emu SAN=1` + LBM_EMU_ASAN=1 runs any of the others the same way."""
     asan = subprocess.run(["/usr/bin/gcc", "-print-file-name=libasan.so"], capture_output=True, text=True).stdout.strip()
     if not os.path.isabs(asan) or not os.path.exists(asan):
         pytest.skip("no libasan next to the system gcc")
@@ -72,7 +74,7 @@ def test_kernels_under_address_sanitizer():
     env = dict(os.environ, LBM_EMU="1", LBM_EMU_ASAN="1", OMP_WAIT_POLICY="passive", LD_PRELOAD=asan,
                ASAN_OPTIONS="detect_leaks=0:abort_on_error=1:verify_asan_link_order=0")
     cmd = [sys.executable, "-m", "pytest", "-m", "gpu", "-q", "-x", "-p", "no:cacheprovider",
-           "tests/test_gpu_two_phase.py", "tests/test_gpu_csf.py", "tests/test_gpu_tp_variants.py"]
+           "tests/test_gpu_two_phase.py", "tests/test_gpu_csf.py", "tests/test_gpu_tp_variants.py", "tests/test_gpu_records_exact.py"]
     r = subprocess.run(cmd, cwd=ROOT, env=env, capture_output=True, text=True, timeout=1500)
     assert r.returncode == 0 and "AddressSanitizer" not in r.stdout + r.stderr, r.stdout[-3000:] + r.stderr[-3000:]
 
@@ -86,7 +88,8 @@ def test_slab_ring_over_the_nccl_stand_in(emu_lib, world, csf_fused="0"):
     r = subprocess.run([sys.executable, os.path.join(EMU_DIR, "ring_threads.py"), str(world)], cwd=ROOT, env=env, capture_output=True,
                        text=True, timeout=900)
     assert r.returncode == 0 and "failures: []" in r.stdout, r.stdout[-3000:] + r.stderr[-3000:]
-    assert r.stdout.count(f"ring of {world}") == 9, r.stdout  # six checks, the two overlapped two-phase runs, the RK diagnostics
+    # six checks, the two overlapped two-phase runs, the RK diagnostics, the statistics and body-force records
+    assert r.stdout.count(f"ring of {world}") == 11, r.stdout
 
 
 @pytest.mark.parametrize("world", [2, 8])
@@ -112,11 +115,12 @@ def test_bench_ring_parity_leg_over_the_nccl_stand_in(emu_lib, world):
 
 def test_blocks_bound_across_ranks_over_the_nccl_stand_in(emu_lib):
     """test/decompose_domain_loop.cpp's four blocks, one per rank (lbm_comm_init_blocks, lbm_link_face_rank,
-    lbm_comm_faces_commit, plain lbm_step): bit-identical to the blocks linked inside one process"""
+    lbm_comm_faces_commit, plain lbm_step), a statistics record on each: bit-identical to the blocks linked inside one process"""
     env = dict(os.environ, OMP_WAIT_POLICY="passive", OMP_NUM_THREADS="1", FAKE_NCCL_TIMEOUT_S="60")
     r = subprocess.run([sys.executable, os.path.join(EMU_DIR, "blocks_ring_threads.py")], cwd=ROOT, env=env, capture_output=True, text=True,
                        timeout=600)
     assert r.returncode == 0 and "bit-exact vs linked blocks = True" in r.stdout, r.stdout[-2000:] + r.stderr[-3000:]
+    assert "statistics record bit-exact vs linked blocks = True" in r.stdout, r.stdout[-2000:]
 
 
 def test_two_phase_halos_behind_the_interior_bands_over_random_rings(emu_lib):

@@ -59,6 +59,36 @@ def test_loop_blocks_vs_oracle(Ln):
         assert np.abs(rho - r).max() < 1e-12 and np.abs(u - orc.calc_u(st[k]["f"], r)).max() < 1e-12
 
 
+def test_loop_blocks_statistics_vs_exact_definition():
+    """a statistics record on the four bound blocks (their face columns are listed nodes in edge columns, the walls of A and
+    C listed rows): each block's record against the exact mean and covariance over the moments of blocks_oracle's run, within
+    test_gpu_records_exact's bound; the region force on block A samples the plain moments its collision uses"""
+    from test_gpu_records_exact import check, moment_delta
+
+    Ln, steps, every = 64, 30, 2
+    orc = Oracle()
+    dom = cases.loop_blocks(Ln, OMEGA)
+    st = BO.init(orc, Ln)
+    rng = np.random.default_rng(7)
+    for k, b in st.items():
+        b["f"] = b["f"] * (1.0 + 0.05 * rng.standard_normal(b["f"].shape))
+        dom[k].set_f(b["f"])
+        dom[k].stats_start(every)
+    order = [dom[k] for k in "ABCD"]
+    samples = {k: [] for k in "ABCD"}
+    delta = {k: np.zeros(3) for k in "ABCD"}
+    for t in range(steps):
+        BO.step(orc, st, Ln, OMEGA)  # leaves rho, u: the moments its collision used
+        if t % every == 0:
+            for k in "ABCD":
+                s = (st[k]["rho"][..., 0], st[k]["u"][..., 0], st[k]["u"][..., 1])
+                samples[k].append(s)
+                delta[k] = np.maximum(delta[k], moment_delta(dom[k].get_f(), s, True, orc))
+        L.step_group(order, 1)
+    for k in "ABCD":
+        check(f"loop block {k}", dom[k].stats(), samples[k], delta[k])
+
+
 def test_loop_blocks_reference_driver_golden():
     """snapshots of the reference's own binary (L = 128, 400 iterations; make_golden.py:case_loop_blocks): the flow the
     body force drives round the channel, m_1 and m_0 of every block"""

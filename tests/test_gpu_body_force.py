@@ -124,27 +124,35 @@ def test_momentum_balance_is_exact(model, slabs):
 
 
 @gpu
-@pytest.mark.parametrize("rules", ["periodic", "cylinder_bb"])
+@pytest.mark.parametrize("rules", ["periodic", "cylinder_bb", "dense"])
 def test_record_matches_numpy_momentum_exchange(rules):
     """1024^2 with 64 discs (125 blocks of links): every step's record equals the definition evaluated by NumPy on the
-    exported state to 1e-13 of the summed magnitudes; with cylinder_bb's inlet, outlet and specular rules present too"""
+    exported state to 1e-13 of the summed magnitudes; with cylinder_bb's inlet, outlet and specular rules present too.
+    dense: 32 x 32 small discs, more than 256 blocks of links, so that every thread of k_body_force_finish sums more than
+    one partial"""
     X = Y = 1024
     steps = 20
     solid = np.zeros((X, Y), dtype=np.uint8)
-    for i in range(8):
-        for j in range(8):
-            solid |= disc(X, Y, 64 + 128 * i + 0.3, 64 + 128 * j + 0.7, 20.5 + i + 0.5 * j)
-    d = L.Domain(L.default_config(X=X, Y=Y, model=L.MODEL_BGK, equilibrium=L.EQ_COMPRESSIBLE, omega=1.6))
-    if rules == "periodic":
-        d.preset_periodic()
+    if rules == "dense":
+        solid = np.tile(disc(32, 32, 15.6, 16.3, 9.2), (32, 32))
     else:
+        for i in range(8):
+            for j in range(8):
+                solid |= disc(X, Y, 64 + 128 * i + 0.3, 64 + 128 * j + 0.7, 20.5 + i + 0.5 * j)
+    d = L.Domain(L.default_config(X=X, Y=Y, model=L.MODEL_BGK, equilibrium=L.EQ_COMPRESSIBLE, omega=1.6))
+    if rules == "cylinder_bb":
         d.preset_free_stream(0.05, 0.0)
+    else:
+        d.preset_periodic()
     d.bc_add_solid(solid)
     d.bc_commit()
     d.set_f(near_equilibrium(X, Y, 5, ux=0.05))
     d.body_force_record(solid, capacity=steps)
     lk = links(solid)
-    assert sum(len(i) for i, _ in lk.values()) > 100 * 256
+    n_links = sum(len(i) for i, _ in lk.values())
+    assert n_links > 100 * 256
+    if rules == "dense":
+        assert n_links > 256 * 256, n_links
     for t in range(steps):
         d.step(1)
         want, scale = momentum_exchange(d.get_f(), lk)
